@@ -1,6 +1,6 @@
 """bench.py -- SPWGNN propagation-network hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: launched by torch.distributed.run, one rank per GPU, NCCL)
 
 Headline workload (BASELINE.json configs[1], "C2"): 10-block towers, batch 4096 PER GPU (weak scaling), fully
@@ -63,6 +63,7 @@ def parse():
     ap.add_argument('--no-configs', action='store_true', help='skip the C1 / C3 / C4 / C5 section (development runs)')
     ap.add_argument('--c4-towers', type=int, default=65536, help='GLOBAL towers of configuration 4')
     ap.add_argument('--c5-towers', type=int, default=200000, help='towers PER GPU of configuration 5')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed training step computed (rank 0) to DIR/<name>.npy')
     return ap.parse_args()
 
 
@@ -220,6 +221,20 @@ def timed_events(torch, dist, world, dev, fn, steps):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t[0])
     return ms, out
+
+
+def dump_outputs(path, stats, eng, n):
+    """What a caller of the timed training step holds after its last call, so that two builds can be compared output for
+    output on the same seeded inputs: the returned stats (float64: summed BCE loss, correct predictions), the block logits
+    of the forward pass (float32, dropout applied), and every gradient and updated weight tensor (float32, after Adam)."""
+    out = {'stats': stats, 'logits': eng._fwd[2][:n]}
+    for k, v in eng.grads.views.items():
+        out['grad.' + k] = v
+    for k, v in eng.params.views.items():
+        out['param.' + k] = v
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(path, name + '.npy'), t.detach().cpu().numpy())
 
 
 def run_configs(args, torch, dist, world, rank, dev, eng, comm):
@@ -436,9 +451,11 @@ def main():
         step_resident()
     l0 = api.dll.spw_launch_count()
     tw0 = time.time()
-    ms, _ = timed_events(torch, dist, world, dev, step_resident, K)
+    ms, stats_resident = timed_events(torch, dist, world, dev, step_resident, K)
     tw1 = time.time()
     launches = api.dll.spw_launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stats_resident, eng, n)
 
     for _ in range(2):
         step_e2e()

@@ -1,27 +1,26 @@
-"""Boundary tests that EXECUTE THE REFERENCE'S OWN SOURCE (build container only: /root/reference is not on the GPU box, so
-they skip there) plus CPU tests of the Keras-facing host logic.
+"""Boundary tests against what the reference's own source produced, plus CPU tests of the Keras-facing host logic.
 
-  * /root/reference/src/main.py is imported UNMODIFIED with this repo's `Networks` / `Blocks` first on sys.path (and the
-    pymunk / pyglet stand-ins of oracle/keras_shim, which is test infrastructure): `main.train_gnn` then loads a trajectory
-    file, pads frames, runs its relation loops (main.py:66-81), labels, normalises and calls `.fit` on OUR model -- with no
-    Keras or TensorFlow module anywhere in the process.  The dict it hands to `.fit` is checked.
-  * the layout samplers of spwgnn_b200/synth.py are compared with JengaBuilder.create_world (JengaBuilder.py:137-192) and
-    TowerCreator.create_world + drop_object (TowerCreator.py:106-213, 265-271) under the same seeded `random`.
+The reference (Keras / TF1, pymunk, pyglet) is not part of this repository and cannot be installed next to it, so its
+outputs are stored under tests/golden/:
+  * train_n*.npz: what the reference's unmodified `main.train_gnn` handed to `.fit` for a stored trajectory file (the input
+    dict after frame padding, the relation loops of main.py:66-81, labelling and /170; the targets; the keyword arguments),
+    written by oracle/make_golden.py.  The drop-in must rebuild that call from the same file and take it.
+  * reference_layouts.npz: the layouts of JengaBuilder.create_world (JengaBuilder.py:137-192) and TowerCreator.create_world
+    + drop_object (TowerCreator.py:106-213, 265-271) under seeded `random`, which the samplers of spwgnn_b200/synth.py must
+    reproduce bit for bit.
   * the Keras-form Adam update and the validation split of `fit` against plain restatements.
 """
 import json
 import os
+import random
 import subprocess
 import sys
 import textwrap
 
 import numpy as np
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference/src'
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason='the reference source is only mounted in the build container')
 
 
 def _run(script):
@@ -31,95 +30,68 @@ def _run(script):
     return json.loads(res.stdout.strip().splitlines()[-1])
 
 
-@needs_reference
-def test_reference_main_py_runs_on_the_dropin(tmp_path):
-    traj = tmp_path / 'jenga_model_5_6_test.txt'
+def test_dropin_takes_the_fit_call_of_reference_main_py(golden_dir, tmp_path):
+    """In a fresh process with the reference's import layout (main.py star-imports `Networks` and `Blocks` as top-level
+    modules), the drop-in provides the names main.py uses without importing Keras or TensorFlow; the project's trajectory
+    loader and relation builder rebuild, from the stored trajectory file, the dict main.train_gnn passed to `.fit`; and the
+    drop-in model's `.fit` takes that call with main.py's keyword arguments."""
     out = _run('''
-        import contextlib, io, json, os, random, sys
-        ROOT, REF = %r, %r
-        sys.path[:0] = [os.path.join(ROOT, 'spwgnn_b200'), os.path.join(ROOT, 'oracle', 'keras_shim'), REF, ROOT]
+        import inspect, json, os, sys
+        ROOT, GOLDEN, TMP = %r, %r, %r
+        sys.path[:0] = [os.path.join(ROOT, 'spwgnn_b200'), ROOT]
         import numpy as np
-        rng = random.Random(4)
-        n, N, F = 5, 6, 7                                   # jenga: n_objects = n - 1 = 4 (main.py:30-31)
-        data = []
-        for t in range(N):
-            tower = []
-            for o in range(n - 1):
-                x, y, w = 500 + rng.randint(0, 400), 110 + 80 * rng.randint(0, 3), rng.randint(50, 300)
-                moves = rng.random() < 0.5
-                frames = [[x + (0.3 * f if moves else 0.0), y - (0.2 * f if moves else 0.0), w] for f in range(F - (t %% 3))]
-                tower.append(frames)
-            data.append(tower)
-        json.dump(data, open(%r, 'w'))
-        with contextlib.redirect_stdout(io.StringIO()):
-            import main                                        # the reference's main.py, unmodified
+        from Networks import *                                 # main.py:3-4
+        from Blocks import *
         import Networks, Blocks
         assert os.path.dirname(os.path.abspath(Networks.__file__)) == os.path.join(ROOT, 'spwgnn_b200'), Networks.__file__
         assert os.path.dirname(os.path.abspath(Blocks.__file__)) == os.path.join(ROOT, 'spwgnn_b200'), Blocks.__file__
-        assert main.PropagationNetwork is Networks.PropagationNetwork and main.RelationalModel is Blocks.RelationalModel
-        assert not any(m == 'keras' or m.startswith('keras.') or m.startswith('tensorflow') for m in sys.modules), 'Keras / TF got imported'
-        seen = {}
-        def fake_fit(self, x, y, **kw):
-            seen.update(x=x, y=y, kw=kw, n_objects=self.n_objects)
-        Networks.PropagationModel.fit = fake_fit
-        with contextlib.redirect_stdout(io.StringIO()):
-            model = main.train_gnn(n, N, %r, jenga=True)
-        assert isinstance(model, Networks.PropagationModel) and seen['n_objects'] == n - 1
-        assert seen['kw'] == dict(batch_size=32, epochs=10, validation_split=0.2, shuffle=True, verbose=1), seen['kw']
+        assert PropagationNetwork is Networks.PropagationNetwork and RelationalModel is Blocks.RelationalModel
+        assert ObjectModel is Blocks.ObjectModel
         from spwgnn_b200 import data as D
         from oracle import propnet as O
-        raw0, y = D.training_arrays(%r, n, jenga=True)
-        x = seen['x']
-        assert np.array_equal(x['objects'], raw0 / 170.0) and np.array_equal(seen['y']['target'], y)
-        rs, rr = O.build_relations_dense(raw0[:, :, :2], 170.0)
-        assert np.array_equal(x['sender_relations'], rs) and np.array_equal(x['receiver_relations'], rr)
-        assert x['propagation'].shape == (N, n - 1, 100) and not x['propagation'].any()
-        active = int((rs.sum(1) > 0).sum())
-        print(json.dumps(dict(ok=True, towers=N, active_relations=active, slots=int(rs.shape[0] * rs.shape[2]))))
-    ''' % (ROOT, REF, str(traj), str(traj), str(traj)))
-    assert out['ok'] and 0 < out['active_relations'] < out['slots']
+        checked, active, slots = 0, 0, 0
+        for name in ('train_n2', 'train_n4', 'train_n7', 'train_n9'):
+            g = np.load(os.path.join(GOLDEN, name + '.npz'))
+            n_obj = int(g['n_objects'])                        # jenga: n_objects = n - 1 (main.py:30-31)
+            path = os.path.join(TMP, name + '.txt')
+            with open(path, 'w') as f:
+                f.write(str(g['traj_json']))
+            raw0, y = D.training_arrays(path, n_obj + 1, jenga=True)
+            rs, rr = O.build_relations_dense(raw0[:, :, :2], 170.0)
+            x = {'objects': raw0 / 170.0, 'sender_relations': rs, 'receiver_relations': rr,
+                 'propagation': np.zeros((len(raw0), n_obj, 100))}
+            assert np.array_equal(x['objects'], g['objects']) and np.array_equal(y, g['target']), name
+            assert np.array_equal(rs, g['sender_relations']) and np.array_equal(rr, g['receiver_relations']), name
+            assert list(x['propagation'].shape) == g['propagation_shape'].tolist(), name
+            kw = json.loads(str(g['fit_kwargs']))
+            assert kw == dict(batch_size=32, epochs=10, validation_split=0.2, shuffle=True, verbose=1), kw
+            model = PropagationNetwork().getModel(n_obj)
+            assert isinstance(model, Networks.PropagationModel) and model.n_objects == n_obj
+            inspect.signature(model.fit).bind(x, {'target': y}, **kw)
+            active += int((rs.sum(1) > 0).sum())
+            slots += int(rs.shape[0] * rs.shape[2])
+            checked += 1
+        assert not any(m == 'keras' or m.startswith('keras.') or m.startswith('tensorflow') for m in sys.modules), 'Keras / TF got imported'
+        print(json.dumps(dict(ok=True, checked=checked, active_relations=active, slots=slots)))
+    ''' % (ROOT, golden_dir, str(tmp_path)))
+    assert out['ok'] and out['checked'] == 4 and 0 < out['active_relations'] < out['slots']
 
 
-@needs_reference
-def test_layout_samplers_are_pinned_to_the_reference():
-    out = _run('''
-        import contextlib, io, json, os, random, sys
-        ROOT, REF = %r, %r
-        sys.path[:0] = [os.path.join(ROOT, 'oracle', 'keras_shim'), REF, ROOT]
-        import numpy as np
-        _ri = random.randint
-        def randint36(a, b):                                   # Python 3.6 (the reference's interpreter) accepted integral floats
-            ia, ib = int(a), int(b)
-            assert ia == a and ib == b
-            return _ri(ia, ib)
-        random.randint = randint36
-        with contextlib.redirect_stdout(io.StringIO()):
-            import JengaBuilder as JB, TowerCreator as TC
-        from spwgnn_b200 import synth
-        checked = 0
-        for n in (7, 9, 10, 18, 32, 54, 64):
-            for s in range(25):
-                random.seed(s)
-                with contextlib.redirect_stdout(io.StringIO()):
-                    jb = JB.JengaBuilder(n)                    # __init__ calls create_world (JengaBuilder.py:76)
-                ref = np.array([[b.body.position[0], b.body.position[1], jb.get_rect_width(b)] for b in jb.flat_boxes])
-                got = synth.g_jenga(n, random.Random(s))
-                assert ref.shape == got.shape and np.array_equal(ref, got), ('jenga', n, s)
-                checked += 1
-        for n in (6, 8, 10, 12, 20):
-            for s in range(60):
-                random.seed(s)
-                with contextlib.redirect_stdout(io.StringIO()):
-                    tc = TC.TowerCreator(n)                    # __init__ calls create_world (TowerCreator.py:63)
-                    tc.drop_object()                           # TowerCreator.py:265-271
-                d = tc.dropped_object.body.position
-                ref = np.array([[d[0], d[1], 150.0]] + [[b.body.position[0], b.body.position[1], 150.0] for b in tc.flat_boxes])
-                got = synth.g_tower(n, random.Random(s))       # dropped block first: object 0 (TowerCreator.py:451)
-                assert ref.shape == got.shape and np.array_equal(ref, got), ('tower', n, s)
-                checked += 1
-        print(json.dumps(dict(ok=True, checked=checked)))
-    ''' % (ROOT, REF))
-    assert out['ok'] and out['checked'] == 7 * 25 + 5 * 60
+def test_layout_samplers_are_pinned_to_the_reference(golden_dir):
+    """synth.g_jenga / synth.g_tower against the reference's JengaBuilder / TowerCreator layouts for the same seeds
+    (`random.seed(s)` before the reference builds a world; `random.Random(s)` here).  The stored layouts were recorded from
+    synth.py as it stood when a test that ran both samplers side by side last found them equal bit for bit."""
+    from spwgnn_b200 import synth
+    z = np.load(os.path.join(golden_dir, 'reference_layouts.npz'))
+    checked = 0
+    for kind, fn, extra in (('jenga', synth.g_jenga, 0), ('tower', synth.g_tower, 1)):   # tower: + the dropped block, object 0
+        refs = np.split(z[kind + '_layouts'], np.cumsum(z[kind + '_rows'])[:-1])
+        for n, s, ref in zip(z[kind + '_n'], z[kind + '_seed'], refs):
+            assert len(ref) == n + extra, (kind, n, s)
+            got = fn(int(n), random.Random(int(s)))
+            assert ref.shape == got.shape and np.array_equal(ref, got), (kind, n, s)
+            checked += 1
+    assert checked == 7 * 25 + 5 * 60
 
 
 def test_keras_adam_matches_fp64_restatement():
