@@ -173,6 +173,15 @@ size_t spw_workspace_bytes(int32_t n_nodes, int32_t n_edges, int training);
  * out[6] = Q and out[7] = Q1, float column-slab [25][n][4] (om layers 1 and 0 after relu, Networks.py:76).               */
 int spw_saved_state_layout(int32_t n_nodes, int32_t n_edges, int64_t* out /*[8]*/);
 
+/* The whole column-slab workspace, exposed for unit tests (tests/test_gpu_stages.py checks every launch of a training step
+ * against an fp64 evaluation of that one launch on the arrays it read).  spw_workspace_layout fills out[0 .. count) and
+ * returns count (SPW_ERR_BAD_ARG if cap < count): first the byte offset of every named array (0 where the mode does not use
+ * the array), then slots, slotsGP (per-step slots of U / S / R / H2S and of [g | p]), bits_rows and bits_floats (rows and
+ * floats of one sign-bit array), edge_stride_floats (floats between the per-step h1 arrays), the two partial strides (floats)
+ * and the workspace size in bytes.  spw_workspace_layout_names gives the comma-separated names in the same order.        */
+const char* spw_workspace_layout_names(void);
+int spw_workspace_layout(int32_t n_nodes, int32_t n_edges, int training, int64_t* out, int cap);
+
 /* Forward (Networks.py:58-96).  obj [n_nodes][3] = [x, y, width]/170 (main.py:91).
  * logits [n_nodes] (channel 0 of the last object-propagator output, Networks.py:94);
  * probs  [n_nodes] sigmoid(logits) or NULL.  training: keep state for spw_backward.

@@ -33,7 +33,7 @@ class SpwGraph(C.Structure):
 
 
 EXPORTS = ['spw_version', 'spw_last_error', 'spw_launch_count', 'spw_profile', 'spw_profile_report', 'spw_ffma_peak', 'spw_tc_selftest', 'spw_tc2_selftest', 'spw_tc_linear', 'spw_csl_linear', 'spw_edges_count', 'spw_edges_fill', 'spw_sample_sizes', 'spw_sample_jenga', 'spw_sample_tower', 'spw_candidates_remove', 'spw_candidates_drop', 'spw_tower_sums', 'spw_workspace_bytes', 'spw_saved_state_layout',
-           'spw_forward', 'spw_bce_grad', 'spw_backward']
+           'spw_workspace_layout_names', 'spw_workspace_layout', 'spw_forward', 'spw_bce_grad', 'spw_backward']
 
 
 class SpwError(RuntimeError):
@@ -91,6 +91,10 @@ class CApi:
         d.spw_workspace_bytes.argtypes = [i32, i32, C.c_int]
         d.spw_saved_state_layout.restype = C.c_int
         d.spw_saved_state_layout.argtypes = [i32, i32, C.POINTER(C.c_int64)]
+        d.spw_workspace_layout_names.restype = C.c_char_p
+        d.spw_workspace_layout_names.argtypes = []
+        d.spw_workspace_layout.restype = C.c_int
+        d.spw_workspace_layout.argtypes = [i32, i32, C.c_int, C.POINTER(C.c_int64), C.c_int]
         d.spw_forward.restype = C.c_int
         d.spw_forward.argtypes = [C.POINTER(SpwParams), C.POINTER(SpwGraph), vp, vp, vp, vp, C.c_size_t, C.c_int,
                                   C.c_float, C.c_uint64, vp]
@@ -103,6 +107,16 @@ class CApi:
     def check(self, rc):
         if rc != 0:
             raise SpwError('libspwgnn error %d: %s' % (rc, self.dll.spw_last_error().decode()))
+
+    def workspace_layout(self, n_nodes, n_edges, training):
+        """spw_workspace_layout as a dict: array name -> byte offset, plus the sizes listed in include/spwgnn.h."""
+        names = self.dll.spw_workspace_layout_names().decode().split(',')
+        out = (C.c_int64 * len(names))()
+        count = self.dll.spw_workspace_layout(n_nodes, n_edges, int(training), out, len(names))
+        if count < 0:
+            self.check(count)
+        assert count == len(names), (count, len(names))
+        return dict(zip(names, [int(v) for v in out]))
 
     @staticmethod
     def params(ptrs):

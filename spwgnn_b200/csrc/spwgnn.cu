@@ -913,6 +913,36 @@ int spw_saved_state_layout(int32_t n_nodes, int32_t n_edges, int64_t* out) {
   return fail(SPW_ERR_UNSUPPORTED, "spw_saved_state_layout: column-slab path only");
 }
 
+// Every named array of the column-slab workspace (byte offsets), then the sizes a reader needs to index them; the order is
+// the one of spw_workspace_layout_names.  Arrays a mode does not use (inference: the backward state) are 0.
+static const char kWorkspaceLayoutNames[] =
+    "W2hi,W2lo,W2Thi,W2Tlo,ENCT,degf,Q1,Q,QV,GP,U,S,R,H2S,PF,PL,X0,X1,X2,C,A,H1,EB,M1,M2,"
+    "dU,dG,T,dS,dR,dH2S,DP,dQ,dQ1,dA,DH1,GB,partE,part0,partN,"
+    "slots,slotsGP,bits_rows,bits_floats,edge_stride_floats,part_stride_floats,part0_stride_floats,total_bytes";
+
+const char* spw_workspace_layout_names(void) { return kWorkspaceLayoutNames; }
+
+int spw_workspace_layout(int32_t n_nodes, int32_t n_edges, int training, int64_t* out, int cap) {
+  if (n_nodes < 0 || n_edges < 0 || !out) return fail(SPW_ERR_BAD_ARG, "spw_workspace_layout: bad argument");
+#if SPW_USE_TC
+  if (use_csl()) {
+    const LayoutC L = make_layout_c(n_nodes, n_edges, training);
+    const size_t offs[] = {L.W2hi, L.W2lo, L.W2Thi, L.W2Tlo, L.ENCT, L.degf, L.Q1, L.Q, L.QV, L.GP, L.U, L.S, L.R, L.H2S, L.PF, L.PL,
+                           L.X0, L.X1, L.X2, L.C, L.A, L.H1, L.EB, L.M1, L.M2, L.dU, L.dG, L.T, L.dS, L.dR, L.dH2S, L.DP, L.dQ, L.dQ1,
+                           L.dA, L.DH1, L.GB, L.partE, L.part0, L.partN};
+    const int64_t sizes[] = {L.slots, L.slotsGP, L.bits_rows, L.bits_floats, (int64_t)kQ150 * n_edges * 4 + 64, (int64_t)L.part_stride,
+                             (int64_t)L.part0_stride, (int64_t)L.total * 4};
+    const int no = (int)(sizeof(offs) / sizeof(offs[0])), ns = (int)(sizeof(sizes) / sizeof(sizes[0]));
+    if (cap < no + ns) return fail(SPW_ERR_BAD_ARG, "spw_workspace_layout: %d entries do not fit in %d", no + ns, cap);
+    for (int i = 0; i < no; ++i) out[i] = (int64_t)offs[i] * 4;
+    for (int i = 0; i < ns; ++i) out[no + i] = sizes[i];
+    return no + ns;
+  }
+#endif
+  (void)training; (void)cap;
+  return fail(SPW_ERR_UNSUPPORTED, "spw_workspace_layout: column-slab path only");
+}
+
 int spw_forward(const SpwParams* w, const SpwGraph* g, const float* obj, float* logits, float* probs, void* workspace,
                 size_t workspace_bytes, int training, float dropout_rate, uint64_t dropout_seed, void* stream) {
   int rc;

@@ -36,6 +36,69 @@ def test_library_is_sm100a_only(built_lib):
     assert 'sm_100a' in out and 'sm_90' not in out and 'sm_80' not in out
 
 
+def _workspace_array_floats(L, n, E):
+    """Floats of every named workspace array, restated from the shapes (column-slab arrays: [quads][rows][4])."""
+    q100, q150, q200 = 26 * n * 4, 38 * n * 4, 50 * n * 4
+    earr = 38 * E * 4 + 64
+    chunks = (E + 31) // 32 + 1
+    bits = L['bits_floats']
+    size = {'W2hi': 24320, 'W2lo': 24320, 'W2Thi': 24320, 'W2Tlo': 24320, 'ENCT': 8 * 24320, 'degf': n,
+            'Q1': q100, 'Q': q100, 'QV': q100, 'GP': q200 * L['slotsGP'], 'U': q100 * L['slots'],
+            'S': q150 * L['slots'], 'R': q150 * L['slots'], 'H2S': q150 * L['slots'], 'PF': chunks * 160, 'PL': chunks * 160,
+            'X0': earr, 'X1': earr, 'X2': earr, 'C': earr, 'A': earr, 'H1': 5 * earr, 'EB': 4 * bits, 'M1': 5 * bits, 'M2': 5 * bits,
+            'dU': 5 * q100, 'dG': 5 * q100, 'T': 4 * q100, 'dS': 4 * q150, 'dR': 4 * q150, 'dH2S': q150, 'DP': q100, 'dQ': q100,
+            'dQ1': q100, 'dA': earr, 'DH1': earr, 'GB': earr, 'partE': 160 * 2 * 160 * 128,
+            'part0': 3 * L['part0_stride_floats'], 'partN': 11 * L['part_stride_floats']}
+    return size
+
+
+@pytest.mark.parametrize('n,E', [(1, 0), (2, 2), (4, 6), (129, 257), (1000, 0), (1000, 8705), (40960, 368640)])
+def test_workspace_layout_hook(built_lib, n, E):
+    """spw_workspace_layout: every array in bounds of spw_workspace_bytes and 16-byte aligned (the TMA tensor maps need it),
+    the training arrays pairwise disjoint, the inference aliases exactly the intended ones, agreement with
+    spw_saved_state_layout.  E = 0 and E = 1 (mod 128) are the edge cases of the sign-bit rows."""
+    import ctypes
+    from spwgnn_b200._capi import CApi
+    api = CApi(built_lib)
+    names = api.dll.spw_workspace_layout_names().decode().split(',')
+    assert len(names) == len(set(names))
+    short = (ctypes.c_int64 * 4)()
+    assert api.dll.spw_workspace_layout(n, E, 1, short, 4) == -1
+    assert api.dll.spw_workspace_layout(-1, E, 1, short, 4) == -1
+    for training in (1, 0):
+        L = api.workspace_layout(n, E, training)
+        total = L['total_bytes']
+        assert total == api.dll.spw_workspace_bytes(n, E, training)
+        assert L['slots'] == (5 if training else 1) and L['slotsGP'] == (5 if training else 2)
+        assert L['bits_rows'] == (E + 127) // 128 * 128 + 128 and L['bits_floats'] == (20 * L['bits_rows'] + 3) // 4
+        assert L['edge_stride_floats'] == 38 * E * 4 + 64
+        size = _workspace_array_floats(L, n, E)
+        backward = ['H1', 'EB', 'M1', 'M2', 'dU', 'dG', 'T', 'dS', 'dR', 'dH2S', 'DP', 'dQ', 'dQ1', 'dA', 'DH1', 'GB', 'partE',
+                    'part0', 'partN']
+        used = [k for k in size if training or k not in backward]
+        if not training:
+            assert all(L[k] == 0 for k in backward)
+            assert L['X0'] == L['X2'] == L['A'] and L['X1'] == L['C'] and L['X0'] != L['X1']
+        spans = {}
+        for k in used:
+            off, nbytes = L[k], 4 * size[k]
+            assert off % 16 == 0, (k, off)
+            assert 0 <= off and off + nbytes <= total, (k, off, nbytes, total)
+            spans[k] = (off, off + nbytes)
+        aliases = set() if training else {frozenset(('X0', 'X2')), frozenset(('X0', 'A')), frozenset(('X2', 'A')), frozenset(('X1', 'C'))}
+        ks = sorted(spans)
+        for i, a in enumerate(ks):
+            for b in ks[i + 1:]:
+                if frozenset((a, b)) in aliases:
+                    continue
+                (a0, a1), (b0, b1) = spans[a], spans[b]
+                assert a1 <= b0 or b1 <= a0, ('overlap', a, spans[a], b, spans[b])
+    saved = (ctypes.c_int64 * 8)()
+    api.check(api.dll.spw_saved_state_layout(n, E, saved))
+    L = api.workspace_layout(n, E, 1)
+    assert list(saved) == [L['bits_rows'], 4 * L['bits_floats'], L['EB'], L['M1'], L['M2'], L['U'], L['Q'], L['Q1']]
+
+
 def test_host_side_argument_checks(built_lib):
     """Errors that are detected before any kernel launch can be exercised without a GPU."""
     import ctypes
