@@ -220,6 +220,52 @@ def _write_record(seconds):
         pass
 
 
+# ---- loss seed (restatement of k_bce_grad's clip) ----------------------------------------------------------------------------
+# k_bce_grad clips at the fp32 constants 1e-7f and 1.f - 1e-7f; the second rounds to 1 - 2^-23 (1 - 1e-7 in double is
+# 1.9e-8 closer to 1, and logits 15.94 .. 16.12 fall between the two)
+CLIP_LO = float(np.float32(1e-7))
+CLIP_HI = float(np.float32(1.0) - np.float32(1e-7))
+
+
+def prob_interval(z):
+    """[p_lo, p_hi] (float64, on z's device) containing the kernels' fp32 p = 1 / (1 + expf(-z)) for fp32 logits z.
+    expf is within 2 ulp of exp(-z) (4 u relative; exact at 0, where it returns 1); the add and the division are correctly
+    rounded, hence monotone, so p lies between the values this arithmetic gives at the smallest and the largest fp32 number
+    expf may return.  Near p = 1 this is the fp32 grid itself (p < 1 - 2^-23 exactly when fl(1 + e) >= 1 + 2^-22, i.e.
+    e >= 3 * 2^-24, z <= ~15.537), which a relative bar on p cannot resolve."""
+    zz = z.detach().cpu().numpy().astype(np.float32)
+    e64 = np.exp(-zz.astype(np.float64))
+    e64 = np.where(zz == 0, 1.0, e64)
+    slack = np.where(zz == 0, 0.0, 4 * U)
+    f32 = np.float32
+    with np.errstate(over='ignore'):
+        lo, hi = e64 * (1 - slack), e64 * (1 + slack)
+        elo = lo.astype(f32)
+        elo = np.where(elo.astype(np.float64) < lo, np.nextafter(elo, f32(np.inf)), elo)
+        ehi = hi.astype(f32)
+        ehi = np.where(ehi.astype(np.float64) > hi, np.nextafter(ehi, f32(0)), ehi)
+        ehi = np.where(hi > np.finfo(f32).max, f32(np.inf), ehi)          # expf may overflow
+        p_hi, p_lo = f32(1) / (f32(1) + elo), f32(1) / (f32(1) + ehi)
+    to = lambda a: torch.from_numpy(a.astype(np.float64)).to(z.device)
+    return to(p_lo), to(p_hi)
+
+
+def bce_seed_reference(z, t, count, got):
+    """fp64 d(mean clipped BCE)/d logit of fp32 logits z with targets t: (ref, absref, ambiguous).  The gradient passes only
+    strictly inside the clip.  `ambiguous` marks the elements whose probability interval (prob_interval) straddles a clip
+    edge, where the kernel's fp32 probability may fall on either side: there the reference follows the branch `got` took
+    (exactly 0 outside, the inside value otherwise).  Everywhere else the branch is fixed."""
+    p = torch.sigmoid(z)
+    p_lo, p_hi = prob_interval(z)
+    inside_sure = (p_lo > CLIP_LO) & (p_hi < CLIP_HI)
+    outside_sure = (p_hi <= CLIP_LO) | (p_lo >= CLIP_HI)
+    amb = ~inside_sure & ~outside_sure
+    inside = torch.where(amb, got.double() != 0, inside_sure)
+    ref = torch.where(inside, (p - t) / count, torch.zeros_like(p))
+    ab = torch.where(inside, (p + (p - t).abs()) / count, torch.zeros_like(p))
+    return ref, ab, amb
+
+
 # ---- dropout masks (restatement of dropout_hash, spw_common.cuh, on the device) -----------------------------------------
 def _keep(seed32, rows, stride, cols, rate, device):
     idx = torch.arange(rows, device=device, dtype=torch.int64)[:, None] * stride + torch.arange(cols, device=device)[None, :]
@@ -405,12 +451,7 @@ def check_step(api, eng, batch, tgt, rate, seed, case):
     ab = terms.abs().sum(1) + Wa['omp.b1'][0]
     chk.bar('logits', logits[:n], ref, ab, 101 * U)
     # loss seed (k_bce_grad): d(mean clipped BCE)/d logit on the GPU's logits
-    z = d64(logits[:n])
-    p = torch.sigmoid(z)
-    t = d64(tgt[:n])
-    inside = (p > 1e-7) & (p < 1 - 1e-7)
-    ref = torch.where(inside, (p - t) / n, torch.zeros_like(p))
-    ab = torch.where(inside, (p + (p - t).abs()) / n, torch.zeros_like(p))
+    ref, ab, _ = bce_seed_reference(d64(logits[:n]), d64(tgt[:n]), n, dl[:n])
     chk.bar('dlogits', dl[:n], ref, ab, 8 * U)
 
     # ================= backward =================
