@@ -32,6 +32,7 @@ extern "C" {
 #define SPW_MAX_NODES 64      /* blocks per tower handled by the edge builder's per-tower CTA */
 #define SPW_N_STEPS 5         /* Networks.py:83 */
 #define SPW_PROP_DIM 100      /* Networks.py:29 */
+#define SPW_SMALL_MAX_NODES 32  /* blocks per tower of the one-CTA-per-tower inference (spw_forward_towers) */
 
 typedef enum {
   SPW_OK = 0,
@@ -191,6 +192,21 @@ int spw_workspace_layout(int32_t n_nodes, int32_t n_edges, int training, int64_t
 int spw_forward(const SpwParams* w, const SpwGraph* g, const float* obj, float* logits, float* probs,
                 void* workspace, size_t workspace_bytes, int training, float dropout_rate,
                 uint64_t dropout_seed, void* stream);
+
+/* Inference with ONE CTA per tower and ONE kernel launch per call: the function of spw_forward(training = 0), for batches of
+ * small towers (a batch-1 predict is about 47 launches through spw_forward).  Plain fp32 FFMA; every sum runs in a fixed
+ * order that depends on the tower alone, so a tower's logits are the same bits whatever else is in the batch and wherever
+ * it sits in it (spw_forward's tiled receiver sums cannot promise that).  Weights are read in the Keras layout of SpwParams.
+ *   max_nodes_per_tower: the caller's max N_t (host value, <= SPW_SMALL_MAX_NODES, else SPW_ERR_UNSUPPORTED); it sizes the
+ *                        shared memory.  A tower with more blocks than that gets NaN logits (and probs) and nothing else
+ *                        of it is written.  Any number of edges per tower (in-degree <= N_t - 1).
+ *   obj [n_nodes][3], logits [n_nodes], probs [n_nodes] or NULL: as spw_forward.
+ *   workspace: at least spw_forward_towers_bytes(n_nodes, n_edges) bytes (the per-edge A_e = c_e.W1a + b1, 152 floats per
+ *              edge), 16-byte aligned; it may be NULL when that size is 0.  Nothing in it is kept after the call.
+ * n_nodes == 0 launches nothing. */
+size_t spw_forward_towers_bytes(int32_t n_nodes, int32_t n_edges);
+int spw_forward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj, float* logits,
+                       float* probs, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Keras binary_crossentropy on probabilities clipped to [1e-7, 1-1e-7] (Networks.py:102), mean over
  * `count` outputs (pass the GLOBAL number of blocks when data-parallel).  Writes dlogits [n_nodes]

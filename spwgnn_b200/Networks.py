@@ -10,7 +10,9 @@ kernels in libspwgnn.so.  Differences by design:
   * logits are exposed (`predict_logits`); `predict_tower_sums` returns the per-tower sum of block
     probabilities the demolish searches use (JengaBuilder.py:254-256, TowerCreator.py:299-300), and
     `score_removals` / `score_drops` run a whole demolish search (candidate towers, scores, argmin)
-    as one packed inference instead of N or 100 batch-1 predicts.
+    as one packed inference instead of N or 100 batch-1 predicts;
+  * `PropagationNetwork(small_batches=True)` sends inference on small batches of small towers through
+    `Engine.forward_towers` (one CTA per tower, one launch) instead of the tiled `Engine.forward`.
 """
 import os
 import sys
@@ -47,10 +49,26 @@ class History:
 class PropagationNetwork:
     """Networks.py:12-104.  Holds the shared weights (one Engine, created when a model first computes) and a per-N facade
     cache like the reference's `self.Nets`; `relnet / objnet / relnetp / objnetp` are the four shared MLPs (Networks.py:40-56)
-    as Blocks descriptors."""
+    as Blocks descriptors.
 
-    def __init__(self, device='cuda', seed=0):
+    small_batches=True: every inference call of the models (predict, predict_logits, predict_towers, predict_tower_sums,
+    score_removals, score_drops, evaluate and the validation pass of fit / fit_towers) uses Engine.forward_towers when the
+    batch's towers have at most `small_max_nodes` blocks and there are at most `small_max_towers` of them, and the tiled
+    Engine.forward otherwise.  Training is unchanged.  On that path a tower's probabilities do not depend on the rest of the
+    batch, bit for bit: a packed demolish search (score_removals, score_drops) gives exactly the sums of one batch-1 predict
+    per candidate.  Off by default: the two paths agree to fp32 rounding, not bit for bit, and the tiled path is faster."""
+
+    # The limits keep forward_towers where its cost stays within about 2x of the tiled path.  It wins nowhere yet: measured
+    # on one B200 at a 1000 W power limit (tools/bench_small.py, profiles/small_r05.json), device time per call, tiled vs
+    # forward_towers: C1 (8-block TowerCreator towers) 248 vs 408 us at 1 tower, 276 vs 402 us at 32; fully connected 10-block
+    # towers 249 vs 533 us at 1, 281 vs 530 us at 128, then 385 vs 2097 us at 512 and 883 vs 7385 us at 2048; one fully
+    # connected tower of 16 / 24 / 32 blocks 249 vs 1194 / 2548 / 4366 us.  What the flag buys is batch invariance.
+    small_max_nodes = 10
+    small_max_towers = 128
+
+    def __init__(self, device='cuda', seed=0, small_batches=False):
         self.Nets = {}
+        self.small_batches = bool(small_batches)
         self.set_weights = False
         self._device, self._seed = device, seed
         self._engine = None
@@ -95,6 +113,14 @@ class PropagationModel:
         return self.network.engine
 
     # ---- inference -----------------------------------------------------------------------------
+    def _infer(self, batch, want_probs=True):
+        """The inference forward of every call below: forward_towers for small batches of small towers when the network
+        was built with small_batches=True, the tiled forward otherwise."""
+        net, eng = self.network, self.engine
+        if net.small_batches and batch.max_nodes <= net.small_max_nodes and batch.n_towers <= net.small_max_towers:
+            return eng.forward_towers(batch, want_probs=want_probs)
+        return eng.forward(batch, training=False, want_probs=want_probs)
+
     def _batch_from_dict(self, x, sel=None):
         obj = np.asarray(x['objects'])
         rs, rr = np.asarray(x['sender_relations']), np.asarray(x['receiver_relations'])
@@ -109,12 +135,12 @@ class PropagationModel:
         the all-zero 'propagation' seed is implied and ignored).  Returns float32 (B, N, 1)."""
         B, N = np.asarray(x['objects']).shape[:2]
         batch = self._batch_from_dict(x)
-        _, probs = self.engine.forward(batch, training=False)
+        _, probs = self._infer(batch)
         return probs.reshape(B, N, 1).cpu().numpy()
 
     def predict_logits(self, x):
         B, N = np.asarray(x['objects']).shape[:2]
-        logits, _ = self.engine.forward(self._batch_from_dict(x), training=False)
+        logits, _ = self._infer(self._batch_from_dict(x))
         return logits.reshape(B, N, 1).cpu().numpy()
 
     def predict_towers(self, towers, inference_glue=True, thr=REL_THRESHOLD, fully_connected=False):
@@ -123,7 +149,7 @@ class PropagationModel:
         (positions/170 thresholded against 170, i.e. fully connected).  Returns a list of (N_t,) arrays."""
         batch = TowerBatch.from_towers(towers, thr=thr, fully_connected=fully_connected,
                                        inference_glue=inference_glue, device=self.engine.device)
-        _, probs = self.engine.forward(batch, training=False)
+        _, probs = self._infer(batch)
         p = probs.cpu().numpy()
         off = batch.node_off_host
         return [p[off[t]:off[t + 1]] for t in range(batch.n_towers)]
@@ -141,13 +167,13 @@ class PropagationModel:
     def predict_tower_sums(self, towers, **kw):
         """Per-tower sum of block probabilities (the demolish searches' score, JengaBuilder.py:254-256), computed on the GPU."""
         batch = TowerBatch.from_towers(towers, device=self.engine.device, **kw)
-        _, probs = self.engine.forward(batch, training=False)
+        _, probs = self._infer(batch)
         return self._tower_sums(batch, probs, want_argmin=False)[0].cpu().numpy()
 
     def _score_candidates(self, obj, pos, n_cand, n_each, inference_glue, thr):
         node_off = np.arange(n_cand + 1, dtype=np.int64) * n_each
         batch = TowerBatch.from_poses(obj, node_off, pos, thr=thr, fully_connected=False, device=self.engine.device, max_nodes=n_each)
-        _, probs = self.engine.forward(batch, training=False)
+        _, probs = self._infer(batch)
         sums, amin = self._tower_sums(batch, probs)
         return sums.cpu().numpy(), int(amin.item())
 
@@ -196,7 +222,7 @@ class PropagationModel:
 
     def test_on_batch(self, batch, target):
         eng = self.engine
-        logits, _ = eng.forward(batch, training=False, want_probs=False)
+        logits, _ = self._infer(batch, want_probs=False)
         _, stats = eng.bce_seed(logits, target, max(batch.n_nodes, 1))
         s = stats.cpu().numpy() / max(batch.n_nodes, 1)
         return float(s[0]), float(s[1])

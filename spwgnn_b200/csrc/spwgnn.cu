@@ -10,6 +10,7 @@
 #include "spw_csl.cuh"
 #include "spw_csl_kernels.cuh"
 #include "spw_csl_wgrad.cuh"
+#include "spw_small.cuh"
 
 #include <stdarg.h>
 #include <stdio.h>
@@ -1115,6 +1116,38 @@ int spw_forward(const SpwParams* w, const SpwGraph* g, const float* obj, float* 
     }
   }
   return check_launch("spw_forward");
+}
+
+size_t spw_forward_towers_bytes(int32_t n_nodes, int32_t n_edges) {
+  if (n_nodes < 0 || n_edges < 0) return 0;
+  return (size_t)n_edges * kDEP * sizeof(float);        // A_e = c_e.W1a + b1, one 152-float row per edge
+}
+
+int spw_forward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj, float* logits,
+                       float* probs, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_forward_towers")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (max_nodes_per_tower < 0) return fail(SPW_ERR_BAD_ARG, "spw_forward_towers: negative max_nodes_per_tower");
+  if (max_nodes_per_tower > SPW_SMALL_MAX_NODES)
+    return fail(SPW_ERR_UNSUPPORTED, "spw_forward_towers: %d blocks in a tower, limit is %d", max_nodes_per_tower, SPW_SMALL_MAX_NODES);
+  const int n = g->n_nodes, E = g->n_edges;
+  if (n == 0 || g->n_towers == 0) return SPW_OK;
+  if (!obj || !logits) return fail(SPW_ERR_BAD_ARG, "spw_forward_towers: null pointer");
+  if (!aligned16(obj) || !aligned16(logits) || (probs && !aligned16(probs)))
+    return fail(SPW_ERR_BAD_ARG, "spw_forward_towers: obj, logits or probs not 16-byte aligned");
+  const size_t need = spw_forward_towers_bytes(n, E);
+  if (workspace_bytes < need) return fail(SPW_ERR_WORKSPACE, "spw_forward_towers: workspace %zu < %zu bytes", workspace_bytes, need);
+  if (need > 0 && (!workspace || !aligned16(workspace)))
+    return fail(SPW_ERR_BAD_ARG, "spw_forward_towers: workspace null or not 16-byte aligned");
+  TowerFwdArgs a;
+  a.w = *w; a.node_off = g->node_off; a.in_off = g->in_off; a.in_snd = g->in_snd; a.in_rcv = g->in_rcv; a.obj = obj;
+  a.logits = logits; a.probs = probs; a.A = reinterpret_cast<float*>(workspace); a.n_edges = E;
+  a.max_nodes = max_nodes_per_tower > 0 ? max_nodes_per_tower : 1;
+  const size_t smem = small_smem_bytes(a.max_nodes);
+  set_smem(k_tower_forward, smem);
+  SPW_KLAUNCH("k_tower_forward", k_tower_forward, dim3(g->n_towers), dim3(kSmallThreads), smem, (cudaStream_t)stream, a);
+  return check_launch("spw_forward_towers");
 }
 
 int spw_bce_grad(const float* logits, const float* target, int32_t n_nodes, double count, float* dlogits, double* stats,

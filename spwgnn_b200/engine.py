@@ -13,6 +13,8 @@ from ._lib import lib, require_cuda, SpwError
 from .graph import TowerBatch, _stream_ptr
 from .params import ParamBuffer, FLAT_SIZE, STATS_TAIL
 
+SMALL_MAX_NODES = 32      # SPW_SMALL_MAX_NODES (include/spwgnn.h): blocks per tower of forward_towers
+
 
 class Workspace:
     """Grow-only device scratch shared by forward and backward (caller-owned, see spwgnn.h)."""
@@ -55,6 +57,7 @@ class Engine:
         self.ws = Workspace(self.device)        # training: must survive until backward
         self.ws_inf = Workspace(self.device)    # inference: separate, so a predict() between forward and
                                                 # backward of a training step cannot clobber saved state
+        self.ws_small = Workspace(self.device)  # forward_towers: separate from both for the same reason
         self._adam = None
         self._fwd = None
         # small inference batches are launch-bound (~60 launches for microseconds of work: the reference's GUI loops predict
@@ -123,6 +126,23 @@ class Engine:
                                           _stream_ptr(self.device)))
         if training:
             self._fwd = (batch, ws, logits, float(dropout_rate))
+        return logits[:n], (probs[:n] if want_probs else None)
+
+    def forward_towers(self, batch: TowerBatch, want_probs=True):
+        """Inference with one CTA per tower in ONE kernel launch (spw_forward_towers): the function of `forward(training=False)`
+        for towers of at most SMALL_MAX_NODES blocks, computed in plain fp32 with every sum in a fixed order.  A tower's
+        results are the same bits whatever else is in the batch.  Returns (logits[:n], probs[:n] or None)."""
+        if batch.max_nodes > SMALL_MAX_NODES:
+            raise SpwError('forward_towers: towers of up to %d blocks, this batch allows %d' % (SMALL_MAX_NODES, batch.max_nodes))
+        api, n = self.api, batch.n_nodes
+        with torch.cuda.device(self.device):
+            logits = torch.empty(max(n, 1), dtype=torch.float32, device=self.device)
+            probs = torch.empty(max(n, 1), dtype=torch.float32, device=self.device) if want_probs else None
+            ws = self.ws_small.get(api.dll.spw_forward_towers_bytes(n, batch.n_edges))
+            wp = self.params.c_struct()
+            api.check(api.dll.spw_forward_towers(ctypes.byref(wp), ctypes.byref(batch.c_graph), int(batch.max_nodes),
+                                                 batch.obj.data_ptr(), logits.data_ptr(), probs.data_ptr() if want_probs else None,
+                                                 ws.data_ptr(), ws.numel(), _stream_ptr(self.device)))
         return logits[:n], (probs[:n] if want_probs else None)
 
     # ---- loss seed + backward -------------------------------------------------------------------
