@@ -222,6 +222,14 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
                  void* workspace, size_t workspace_bytes, const SpwParams* grads, float dropout_rate,
                  void* stream);
 
+/* Gradient of sum_i dlogits[i]*logit[i] with respect to obj [n_nodes][3] ([x, y, width]/170), the relations of g held
+ * fixed, written (not accumulated) to dobj [n_nodes][3] (16-byte aligned).  No weight gradient is computed.
+ * workspace / dropout_rate: as spw_backward (the workspace of a training spw_forward, passed untouched; the rate of that
+ * forward); the forward state in it is left unchanged.  Deterministic: every sum runs in a fixed order that depends on the
+ * tower alone.  n_nodes == 0 launches nothing.  SPW_ERR_UNSUPPORTED on the round-1 data path (SPW_CSL=0). */
+int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                     size_t workspace_bytes, float dropout_rate, float* dobj, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

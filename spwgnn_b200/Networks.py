@@ -12,7 +12,8 @@ kernels in libspwgnn.so.  Differences by design:
     `score_removals` / `score_drops` run a whole demolish search (candidate towers, scores, argmin)
     as one packed inference instead of N or 100 batch-1 predicts;
   * `PropagationNetwork(small_batches=True)` sends inference on small batches of small towers through
-    `Engine.forward_towers` (one CTA per tower, one launch) instead of the tiled `Engine.forward`.
+    `Engine.forward_towers` (one CTA per tower, one launch) instead of the tiled `Engine.forward`;
+  * `stability_gradients` differentiates each tower's demolish score with respect to its block poses.
 """
 import os
 import sys
@@ -21,13 +22,13 @@ import numpy as np
 import torch
 
 try:
-    from .engine import Engine
+    from .engine import Engine, PropNetObjFunction
     from .graph import TowerBatch, REL_THRESHOLD
     from ._lib import SpwError
     from .Blocks import RelationalModel, ObjectModel
 except ImportError:      # imported as top-level `Networks` (reference style: `from Networks import *`)
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    from spwgnn_b200.engine import Engine
+    from spwgnn_b200.engine import Engine, PropNetObjFunction
     from spwgnn_b200.graph import TowerBatch, REL_THRESHOLD
     from spwgnn_b200._lib import SpwError
     from spwgnn_b200.Blocks import RelationalModel, ObjectModel
@@ -209,6 +210,26 @@ class PropagationModel:
             api.check(api.dll.spw_candidates_drop(raw.data_ptr(), N, ps.data_ptr(), K, float(width), obj.data_ptr(), pos.data_ptr(),
                                                   int(bool(inference_glue)), torch.cuda.current_stream(dev).cuda_stream))
         return self._score_candidates(obj[:K * (N + 1)], pos[:K * (N + 1)], K, N + 1, inference_glue, thr)
+
+    def stability_gradients(self, towers, inference_glue=True, thr=REL_THRESHOLD, fully_connected=False):
+        """Gradient of each tower's demolish score sum_i p_i (JengaBuilder.py:254-256) with respect to its blocks' RAW
+        [x, y, width]: a list of (N_t, 3) float64 arrays, in pixels.  `towers` and the relation options are those of
+        predict_towers; the relations are held fixed (they come from a distance threshold, which is piecewise constant).
+        Towers are independent, so one packed backward pass of the batch's total gives every tower the gradient of its own
+        sum.  p = sigmoid(logits) in fp32; the factor 1/170 of the feature normalisation is applied in float64.  Always the
+        tiled path (PropNetObjFunction): the per-tower kernel of small_batches=True has no backward pass."""
+        if not towers:
+            return []
+        eng = self.engine
+        batch = TowerBatch.from_towers(towers, thr=thr, fully_connected=fully_connected, inference_glue=inference_glue,
+                                       device=eng.device)
+        obj = batch.obj.detach().clone().requires_grad_(True)
+        with torch.enable_grad():
+            p = torch.sigmoid(PropNetObjFunction.apply(obj, eng, batch))
+            (g,) = torch.autograd.grad(p.sum(), [obj])
+        g = g.cpu().numpy().astype(np.float64) / REL_THRESHOLD
+        off = batch.node_off_host
+        return [g[off[t]:off[t + 1]] for t in range(batch.n_towers)]
 
     # ---- training ------------------------------------------------------------------------------
     def train_on_batch(self, batch, target):

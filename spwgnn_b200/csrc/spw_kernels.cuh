@@ -813,6 +813,7 @@ struct EdgeEncBwdArgs {
   float inv_keep;           // 1/(1-rate) of the dropout applied to c_e in the forward pass (1 if none)
   float* partM;             // [gridDim.x][4][160*160]: W1A, RM3, RM2, RM1
   float* part0;             // [gridDim.x][3][152]: d rm.w0 row 0, row 1, d rm.b0
+  float* G0;                // [E][152] or null: the gradient w.r.t. the pre-activation of rm layer 0 (columns 0..149; spw_backward_obj)
 };
 
 constexpr int kTMB = 64;    // rows per tile in the encoder backward (5 resident activation tiles)
@@ -886,6 +887,11 @@ __global__ void __launch_bounds__(kThreads, 1) k_edge_encode_bwd(EdgeEncBwdArgs 
       if (first) { part0[k] = g0; part0[kDEP + k] = g1; part0[2 * kDEP + k] = gb; }
       else { part0[k] += g0; part0[kDEP + k] += g1; part0[2 * kDEP + k] += gb; }
     }
+    if (a.G0)
+      for (int idx = tid; idx < rows * kDE; idx += kThreads) {
+        const int r = idx / kDE, k = idx - r * kDE;
+        a.G0[(size_t)(e0 + r) * kDEP + k] = Bd[(size_t)r * kDEP + k];
+      }
     first = false;
     __syncthreads();
   }

@@ -11,6 +11,7 @@
 #include "spw_csl_kernels.cuh"
 #include "spw_csl_wgrad.cuh"
 #include "spw_small.cuh"
+#include "spw_obj_grad.cuh"
 
 #include <stdarg.h>
 #include <stdio.h>
@@ -1160,21 +1161,14 @@ int spw_bce_grad(const float* logits, const float* target, int32_t n_nodes, doub
   return check_launch("spw_bce_grad");
 }
 
-int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
-                 size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream) {
-  int rc;
-  if ((rc = check_params(w, "spw_backward(weights)")) != SPW_OK) return rc;
-  if ((rc = check_params(grads, "spw_backward(grads)")) != SPW_OK) return rc;
-  if ((rc = check_graph(g)) != SPW_OK) return rc;
+}  // extern "C"
+
+namespace {
+// The backward pass of the row-major data path (round 1; the only one of the FFMA build).  grads == null (spw_backward_obj):
+// no weight gradient is reduced; dobj != null: d obj [n][3] from the layer-0 gradients (k_obj_grad_c, spw_obj_grad.cuh).
+int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                  size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream, float* dobj) {
   const int n = g->n_nodes, E = g->n_edges;
-  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward: bad workspace");
-  if (dropout_rate < 0.f || dropout_rate >= 1.f) return fail(SPW_ERR_BAD_ARG, "spw_backward: dropout rate %g outside [0,1)", dropout_rate);
-#if SPW_USE_TC
-  if (use_csl() && n > 0) {
-    if (!obj || !dlogits) return fail(SPW_ERR_BAD_ARG, "spw_backward: null pointer");
-    return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, grads, dropout_rate, (cudaStream_t)stream);
-  }
-#endif
   const float inv_keep = dropout_rate > 0.f ? 1.f / (1.f - dropout_rate) : 1.f;
   const Layout L = make_layout(n, E, 1);
   if (workspace_bytes < L.total * sizeof(float))
@@ -1183,7 +1177,7 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
   float* ws = reinterpret_cast<float*>(workspace);
   auto PK = [&](int id) { return ws + L.pack[id]; };
   const size_t nP = (size_t)n * kDP, nE = (size_t)n * kDEP;
-  if (n == 0) {
+  if (n == 0 && grads) {
     // no data: all gradients are zero
     static const int sizes[22] = {300, 22500, 22500, 22500, 150, 150, 150, 150, 200, 10000, 100, 100,
                                   52500, 22500, 15000, 150, 150, 100, 30000, 10100, 100, 101};
@@ -1293,26 +1287,28 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
 
   // ---- node-level weight gradients, each one contraction over all steps' rows -------------------
   const float* degf = ws + L.degf;
-  // omp layer 0 = [V1a; V1b; V1c], bias c1
-  launch_wgrad(st, 5 * n, ws + L.Q, kDP, kDP, n, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 0, 0, grads->omp_b[0], 0});
-  launch_wgrad(st, 5 * n, ws + L.G, kDP, kDP, 0, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 100, 0, nullptr, 0});
-  launch_wgrad(st, 5 * n, ws + L.P, kDP, kDP, 0, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 200, 0, nullptr, 0});
-  // omp layer 1: channels 1..100 from T (steps 1..4), channel 0 from the head
-  launch_wgrad(st, 4 * n, ws + L.U, kDP, kDP, 0, nullptr, 0, ws + L.T, kDP, kDP, partN, {grads->omp_w[1], 101, 0, 1, grads->omp_b[1], 1});
-  launch_wgrad(st, n, U5, kDP, kDP, 0, nullptr, 0, dlogits, 1, 1, partN, {grads->omp_w[1], 101, 0, 0, grads->omp_b[1], 0});
-  // rmp layer 2 (W3, b3 scaled by in-degree)
-  launch_wgrad(st, 5 * n, ws + L.H2S, kDEP, kDE, 0, degf, n, ws + L.dG, kDP, kDP, partN, {grads->rmp_w[2], 100, 0, 0, grads->rmp_b[2], 0});
-  // rmp layer 0 rows 150..349 (W1b, W1c): X = p^{l} for steps 2..5
-  launch_wgrad(st, 4 * n, ws + L.P + nP, kDP, kDP, 0, nullptr, 0, ws + L.dS, kDEP, kDE, partN, {grads->rmp_w[0], 150, 150, 0, nullptr, 0});
-  launch_wgrad(st, 4 * n, ws + L.P + nP, kDP, kDP, 0, nullptr, 0, ws + L.dR, kDEP, kDE, partN, {grads->rmp_w[0], 150, 250, 0, nullptr, 0});
-  // object encoder
-  launch_wgrad(st, n, ws + L.Q1, kDP, kDP, 0, nullptr, 0, ws + L.dQ, kDP, kDP, partN, {grads->om_w[1], 100, 0, 0, grads->om_b[1], 0});
+  if (grads) {
+    // omp layer 0 = [V1a; V1b; V1c], bias c1
+    launch_wgrad(st, 5 * n, ws + L.Q, kDP, kDP, n, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 0, 0, grads->omp_b[0], 0});
+    launch_wgrad(st, 5 * n, ws + L.G, kDP, kDP, 0, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 100, 0, nullptr, 0});
+    launch_wgrad(st, 5 * n, ws + L.P, kDP, kDP, 0, nullptr, 0, ws + L.dU, kDP, kDP, partN, {grads->omp_w[0], 100, 200, 0, nullptr, 0});
+    // omp layer 1: channels 1..100 from T (steps 1..4), channel 0 from the head
+    launch_wgrad(st, 4 * n, ws + L.U, kDP, kDP, 0, nullptr, 0, ws + L.T, kDP, kDP, partN, {grads->omp_w[1], 101, 0, 1, grads->omp_b[1], 1});
+    launch_wgrad(st, n, U5, kDP, kDP, 0, nullptr, 0, dlogits, 1, 1, partN, {grads->omp_w[1], 101, 0, 0, grads->omp_b[1], 0});
+    // rmp layer 2 (W3, b3 scaled by in-degree)
+    launch_wgrad(st, 5 * n, ws + L.H2S, kDEP, kDE, 0, degf, n, ws + L.dG, kDP, kDP, partN, {grads->rmp_w[2], 100, 0, 0, grads->rmp_b[2], 0});
+    // rmp layer 0 rows 150..349 (W1b, W1c): X = p^{l} for steps 2..5
+    launch_wgrad(st, 4 * n, ws + L.P + nP, kDP, kDP, 0, nullptr, 0, ws + L.dS, kDEP, kDE, partN, {grads->rmp_w[0], 150, 150, 0, nullptr, 0});
+    launch_wgrad(st, 4 * n, ws + L.P + nP, kDP, kDP, 0, nullptr, 0, ws + L.dR, kDEP, kDE, partN, {grads->rmp_w[0], 150, 250, 0, nullptr, 0});
+    // object encoder
+    launch_wgrad(st, n, ws + L.Q1, kDP, kDP, 0, nullptr, 0, ws + L.dQ, kDP, kDP, partN, {grads->om_w[1], 100, 0, 0, grads->om_b[1], 0});
+  }
   {
     RowsSeg s = {ws + L.dQ, kDP, kDP};
     LinOpt o; o.mulsrc = ws + L.Q1; o.ld_mul = kDP; o.mulmode = 1;
     run_linear(st, ws, L, {T_OM1T, P_OM1T, 0}, n, kDP, 1, &s, ws + L.dQ1, kDP, o);
   }
-  launch_wgrad(st, n, obj + 1, 3, 2, 0, nullptr, 0, ws + L.dQ1, kDP, kDP, partN, {grads->om_w[0], 100, 0, 0, grads->om_b[0], 0});
+  if (grads) launch_wgrad(st, n, obj + 1, 3, 2, 0, nullptr, 0, ws + L.dQ1, kDP, kDP, partN, {grads->om_w[0], 100, 0, 0, grads->om_b[0], 0});
 
   // ---- edge-level weight gradients --------------------------------------------------------------
   if (E > 0) {
@@ -1320,7 +1316,7 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
 #if SPW_USE_TC
     launch_reduce(st, ws + L.partE, egrid, (int)tc::kWgPartFloats, 0, -1, tc::kWgFeat1, kDE, kDE, {grads->rmp_w[1], 150, 0, 0, grads->rmp_b[1], 0});
 #else
-    launch_reduce(st, ws + L.partE, egrid, 160 * 160, 0, 10, 10, kDE, kDE, {grads->rmp_w[1], 150, 0, 0, grads->rmp_b[1], 0});
+    if (grads) launch_reduce(st, ws + L.partE, egrid, 160 * 160, 0, 10, 10, kDE, kDE, {grads->rmp_w[1], 150, 0, 0, grads->rmp_b[1], 0});
 #endif
 #if SPW_USE_TC
     {   // relation-encoder backward, layer by layer on the tensor cores (activations X0, X1, X2, C saved by the forward pass)
@@ -1359,18 +1355,20 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
     a.RM1 = PK(P_RM1); a.RM2 = PK(P_RM2); a.RM3 = PK(P_RM3); a.b1 = w->rm_b[1]; a.b2 = w->rm_b[2]; a.b3 = w->rm_b[3];
     a.RM1T = PK(P_RM1T); a.RM2T = PK(P_RM2T); a.RM3T = PK(P_RM3T); a.W1AT = PK(P_W1AT); a.dA = ws + L.dA;
     a.X1 = ws + L.EX1; a.X2 = ws + L.EX2; a.C = ws + L.EC; a.inv_keep = inv_keep;
-    a.partM = ws + L.partM; a.part0 = ws + L.part0;
+    a.partM = ws + L.partM; a.part0 = ws + L.part0; a.G0 = dobj ? ws + L.GB : nullptr;
     set_smem(k_edge_encode_bwd, edge_encb_smem());
     SPW_KLAUNCH("k_edge_encode_bwd", k_edge_encode_bwd, dim3(bgrid), dim3(kThreads), edge_encb_smem(), st, a);
-    const int ps = 4 * 160 * 160;
-    launch_reduce(st, ws + L.partM, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rmp_w[0], 150, 0, 0, grads->rmp_b[0], 0});
-    launch_reduce(st, ws + L.partM + 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[3], 150, 0, 0, grads->rm_b[3], 0});
-    launch_reduce(st, ws + L.partM + 2 * 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[2], 150, 0, 0, grads->rm_b[2], 0});
-    launch_reduce(st, ws + L.partM + 3 * 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[1], 150, 0, 0, grads->rm_b[1], 0});
-    // layer 0: part0 rows [w0 row 0 | w0 row 1 | b0], each kDEP long  ->  treat as Kin = 2 (+ bias row)
-    launch_reduce(st, ws + L.part0, bgrid, 3 * kDEP, kDEP, 0, 0, 2, kDE, {grads->rm_w[0], 150, 0, 0, grads->rm_b[0], 0});
+    if (grads) {
+      const int ps = 4 * 160 * 160;
+      launch_reduce(st, ws + L.partM, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rmp_w[0], 150, 0, 0, grads->rmp_b[0], 0});
+      launch_reduce(st, ws + L.partM + 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[3], 150, 0, 0, grads->rm_b[3], 0});
+      launch_reduce(st, ws + L.partM + 2 * 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[2], 150, 0, 0, grads->rm_b[2], 0});
+      launch_reduce(st, ws + L.partM + 3 * 160 * 160, bgrid, ps, 0, 10, 10, kDE, kDE, {grads->rm_w[1], 150, 0, 0, grads->rm_b[1], 0});
+      // layer 0: part0 rows [w0 row 0 | w0 row 1 | b0], each kDEP long  ->  treat as Kin = 2 (+ bias row)
+      launch_reduce(st, ws + L.part0, bgrid, 3 * kDEP, kDEP, 0, 0, 2, kDE, {grads->rm_w[0], 150, 0, 0, grads->rm_b[0], 0});
+    }
 #endif
-  } else {
+  } else if (grads) {
     cudaMemsetAsync(grads->rmp_w[1], 0, 22500 * sizeof(float), st);
     cudaMemsetAsync(grads->rmp_b[1], 0, 150 * sizeof(float), st);
     cudaMemsetAsync(grads->rmp_w[0], 0, 150 * 150 * sizeof(float), st);   // rows 0..149 (rows 150.. written above)
@@ -1380,7 +1378,52 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
       cudaMemsetAsync(grads->rm_b[i], 0, 150 * sizeof(float), st);
     }
   }
-  return check_launch("spw_backward");
+  if (dobj) {   // d obj from D_e (k_edge_encode_bwd's layer-0 gradient, in GB) and dQ1 (DESIGN.md section 2)
+    ObjGradArgs a;
+    a.n = n; a.in_off = g->in_off; a.out_off = g->out_off; a.out_pos = g->out_pos;
+    a.G0 = ws + L.GB; a.g_ld = kDEP; a.dQ1 = ws + L.dQ1; a.q_ld = kDP;
+    a.rm_w0 = w->rm_w[0]; a.om_w0 = w->om_w[0]; a.dobj = dobj;
+    SPW_KLAUNCH_PDL("k_obj_grad_c", k_obj_grad_c<false>, dim3(grid_for(n, 256)), dim3(256), 0, st, a);
+  }
+  return check_launch(grads ? "spw_backward" : "spw_backward_obj");
+}
+}  // namespace
+
+extern "C" {
+
+int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                 size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_backward(weights)")) != SPW_OK) return rc;
+  if ((rc = check_params(grads, "spw_backward(grads)")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward: bad workspace");
+  if (dropout_rate < 0.f || dropout_rate >= 1.f) return fail(SPW_ERR_BAD_ARG, "spw_backward: dropout rate %g outside [0,1)", dropout_rate);
+#if SPW_USE_TC
+  if (use_csl() && g->n_nodes > 0) {
+    if (!obj || !dlogits) return fail(SPW_ERR_BAD_ARG, "spw_backward: null pointer");
+    return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, grads, dropout_rate, (cudaStream_t)stream);
+  }
+#endif
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, grads, dropout_rate, stream, nullptr);
+}
+
+int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                     size_t workspace_bytes, float dropout_rate, float* dobj, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_backward_obj")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (g->n_nodes == 0) return SPW_OK;
+  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward_obj: workspace null or not 16-byte aligned");
+  if (!obj || !dlogits || !dobj) return fail(SPW_ERR_BAD_ARG, "spw_backward_obj: null pointer");
+  if (!aligned16(dobj)) return fail(SPW_ERR_BAD_ARG, "spw_backward_obj: dobj not 16-byte aligned");
+  if (dropout_rate < 0.f || dropout_rate >= 1.f) return fail(SPW_ERR_BAD_ARG, "spw_backward_obj: dropout rate %g outside [0,1)", dropout_rate);
+#if SPW_USE_TC
+  if (!use_csl()) return fail(SPW_ERR_UNSUPPORTED, "spw_backward_obj: not implemented on the round-1 data path (SPW_CSL=0)");
+  return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, nullptr, dropout_rate, (cudaStream_t)stream, dobj);
+#else
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj);
+#endif
 }
 
 }  // extern "C"

@@ -232,3 +232,44 @@ class PropNetFunction(torch.autograd.Function):
                            'saved for this one (one Engine keeps one training step in flight)')
         g = ctx.engine.backward(dlogits)
         return g.flat.clone(), None, None
+
+
+class PropNetObjFunction(torch.autograd.Function):
+    """torch.autograd bridge for the gradient with respect to the block features: logits = PropNetObjFunction.apply(obj,
+    engine, batch).  obj: (n, 3) fp32 on the engine's device, [x, y, width] / 170, used in place of batch.obj; the relations
+    of `batch` and the weights are constants (no gradient flows to them, and the weights must not change before backward).
+
+    The forward pass is a training spw_forward at dropout rate 0, whose logits are the inference logits bit for bit, into a
+    workspace owned by this call and kept until the autograd graph is freed.  It never touches Engine.ws, so it does not
+    disturb a training step in flight, and several calls may be in flight at once.  The backward pass is spw_backward_obj:
+    the data gradients of the network without any weight gradient."""
+
+    @staticmethod
+    def forward(ctx, obj, engine, batch):
+        n = batch.n_nodes
+        if obj.shape != (n, 3) or obj.dtype != torch.float32 or obj.device != engine.device:
+            raise SpwError('PropNetObjFunction: obj must be (%d, 3) float32 on %s, got %s %s on %s'
+                           % (n, engine.device, tuple(obj.shape), obj.dtype, obj.device))
+        api = engine.api
+        obj = obj.detach().contiguous()
+        with torch.cuda.device(engine.device):
+            logits = torch.empty(n, dtype=torch.float32, device=engine.device)
+            nbytes = api.dll.spw_workspace_bytes(n, batch.n_edges, 1)
+            ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=engine.device)
+            wp = engine.params.c_struct()
+            api.check(api.dll.spw_forward(ctypes.byref(wp), ctypes.byref(batch.c_graph), obj.data_ptr(), logits.data_ptr(), None,
+                                          ws.data_ptr(), nbytes, 1, 0.0, 0, _stream_ptr(engine.device)))
+        ctx.engine, ctx.batch, ctx.obj, ctx.ws, ctx.nbytes = engine, batch, obj, ws, nbytes
+        return logits
+
+    @staticmethod
+    def backward(ctx, dlogits):
+        engine, batch = ctx.engine, ctx.batch
+        api, n = engine.api, batch.n_nodes
+        dl = dlogits.detach().to(torch.float32).contiguous()
+        with torch.cuda.device(engine.device):
+            dobj = torch.empty(n, 3, dtype=torch.float32, device=engine.device)
+            wp = engine.params.c_struct()
+            api.check(api.dll.spw_backward_obj(ctypes.byref(wp), ctypes.byref(batch.c_graph), ctx.obj.data_ptr(), dl.data_ptr(),
+                                               ctx.ws.data_ptr(), ctx.nbytes, 0.0, dobj.data_ptr(), _stream_ptr(engine.device)))
+        return dobj, None, None
