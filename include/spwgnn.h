@@ -230,6 +230,19 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
 int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
                      size_t workspace_bytes, float dropout_rate, float* dobj, void* stream);
 
+/* Gradient of sum_i dlogits[i]*logit[i] with respect to the relation weights: relation e = (s -> r) gets a weight w_e that
+ * multiplies both of its one-hot entries (sender_relations[s, e] and receiver_relations[r, e] of the reference's dense input),
+ * and drel[e] = d/dw_e at w = 1, the relations of g held in place: the sum of the Keras gradients with respect to those two
+ * entries.  drel [n_edges] (4-byte aligned) is written, not accumulated; drel[k] belongs to the receiver-major relation
+ * in_snd[k] -> in_rcv[k].  The relation o of the sender-major (slot) order, the order of the reference's relation columns
+ * within a tower, is drel[out_pos[o]].  dobj: NULL, or [n_nodes][3] (16-byte aligned) receiving spw_backward_obj's result
+ * bit for bit from the same pass.  No weight gradient is computed.  workspace / dropout_rate: as spw_backward_obj; the
+ * forward state in it is left unchanged.  Deterministic: every sum runs in a fixed order that depends on the tower alone.
+ * n_nodes == 0 launches nothing, and n_edges == 0 launches nothing for drel (drel may then be NULL).  SPW_ERR_UNSUPPORTED
+ * on the round-1 data path (SPW_CSL=0). */
+int spw_backward_rel(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                     size_t workspace_bytes, float dropout_rate, float* drel, float* dobj, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

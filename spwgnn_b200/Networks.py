@@ -13,7 +13,8 @@ kernels in libspwgnn.so.  Differences by design:
     as one packed inference instead of N or 100 batch-1 predicts;
   * `PropagationNetwork(small_batches=True)` sends inference on small batches of small towers through
     `Engine.forward_towers` (one CTA per tower, one launch) instead of the tiled `Engine.forward`;
-  * `stability_gradients` differentiates each tower's demolish score with respect to its block poses.
+  * `stability_gradients` differentiates each tower's demolish score with respect to its block poses, and
+    `relation_gradients` with respect to the weights of its relations (which contacts hold the tower up).
 """
 import os
 import sys
@@ -230,6 +231,35 @@ class PropagationModel:
         g = g.cpu().numpy().astype(np.float64) / REL_THRESHOLD
         off = batch.node_off_host
         return [g[off[t]:off[t + 1]] for t in range(batch.n_towers)]
+
+    def relation_gradients(self, towers, inference_glue=True, thr=REL_THRESHOLD, fully_connected=False):
+        """Gradient of each tower's demolish score sum_i p_i with respect to the weights of its relations: relation e = (s -> r)
+        gets a weight w_e multiplying both of its one-hot entries in the reference's sender_relations / receiver_relations, and
+        the value is d(sum_i p_i)/dw_e at w = 1 (the sum of the Keras gradients with respect to those two entries).  Returns, per
+        tower, (pairs, grads): pairs (E_t, 2) int64 local (sender, receiver) block indices of the tower's active relations in
+        the reference's slot order (main.py:69-81: sender outer, receiver inner), grads (E_t,) float64.  Weights are
+        dimensionless, so no 1/170 factor applies.  `towers` and the relation options are those of predict_towers; one packed
+        pass of Engine.relation_gradients with the seed p (1 - p) serves the whole batch."""
+        if not towers:
+            return []
+        eng = self.engine
+        batch = TowerBatch.from_towers(towers, thr=thr, fully_connected=fully_connected, inference_glue=inference_glue,
+                                       device=eng.device)
+
+        def seed(z):
+            p = torch.sigmoid(z)
+            return p * (1 - p)
+        drel, _ = eng.relation_gradients(batch, seed)
+        E, off = batch.n_edges, batch.node_off_host
+        if E == 0:
+            return [(np.zeros((0, 2), np.int64), np.zeros(0, np.float64)) for _ in range(batch.n_towers)]
+        o = batch.out_pos[:E].long()                      # slot (sender-major) order -> receiver-major row
+        snd = batch.in_snd[:E].long()[o].cpu().numpy()
+        rcv = batch.in_rcv[:E].long()[o].cpu().numpy()
+        val = drel[o].cpu().numpy().astype(np.float64)
+        eo = batch.out_off[:batch.n_nodes + 1].cpu().numpy().astype(np.int64)[off]
+        return [(np.stack([snd[eo[t]:eo[t + 1]], rcv[eo[t]:eo[t + 1]]], 1) - off[t], val[eo[t]:eo[t + 1]])
+                for t in range(batch.n_towers)]
 
     # ---- training ------------------------------------------------------------------------------
     def train_on_batch(self, batch, target):

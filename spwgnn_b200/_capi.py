@@ -33,7 +33,7 @@ class SpwGraph(C.Structure):
 
 
 EXPORTS = ['spw_version', 'spw_last_error', 'spw_launch_count', 'spw_profile', 'spw_profile_report', 'spw_ffma_peak', 'spw_tc_selftest', 'spw_tc2_selftest', 'spw_tc_linear', 'spw_csl_linear', 'spw_edges_count', 'spw_edges_fill', 'spw_sample_sizes', 'spw_sample_jenga', 'spw_sample_tower', 'spw_candidates_remove', 'spw_candidates_drop', 'spw_tower_sums', 'spw_workspace_bytes', 'spw_saved_state_layout',
-           'spw_workspace_layout_names', 'spw_workspace_layout', 'spw_forward', 'spw_forward_towers_bytes', 'spw_forward_towers', 'spw_bce_grad', 'spw_backward', 'spw_backward_obj']
+           'spw_workspace_layout_names', 'spw_workspace_layout', 'spw_forward', 'spw_forward_towers_bytes', 'spw_forward_towers', 'spw_bce_grad', 'spw_backward', 'spw_backward_obj', 'spw_backward_rel']
 
 
 class SpwError(RuntimeError):
@@ -109,6 +109,8 @@ class CApi:
                                    C.POINTER(SpwParams), C.c_float, vp]
         d.spw_backward_obj.restype = C.c_int
         d.spw_backward_obj.argtypes = [C.POINTER(SpwParams), C.POINTER(SpwGraph), vp, vp, vp, C.c_size_t, C.c_float, vp, vp]
+        d.spw_backward_rel.restype = C.c_int
+        d.spw_backward_rel.argtypes = [C.POINTER(SpwParams), C.POINTER(SpwGraph), vp, vp, vp, C.c_size_t, C.c_float, vp, vp, vp]
 
     def check(self, rc):
         if rc != 0:

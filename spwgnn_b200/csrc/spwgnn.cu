@@ -12,6 +12,7 @@
 #include "spw_csl_wgrad.cuh"
 #include "spw_small.cuh"
 #include "spw_obj_grad.cuh"
+#include "spw_rel_grad.cuh"
 
 #include <stdarg.h>
 #include <stdio.h>
@@ -1165,9 +1166,10 @@ int spw_bce_grad(const float* logits, const float* target, int32_t n_nodes, doub
 
 namespace {
 // The backward pass of the row-major data path (round 1; the only one of the FFMA build).  grads == null (spw_backward_obj):
-// no weight gradient is reduced; dobj != null: d obj [n][3] from the layer-0 gradients (k_obj_grad_c, spw_obj_grad.cuh).
+// no weight gradient is reduced; dobj != null: d obj [n][3] from the layer-0 gradients (k_obj_grad_c, spw_obj_grad.cuh);
+// drel != null: d drel [E] with respect to the relation weights (k_rel_grad_step / k_rel_grad_enc, spw_rel_grad.cuh).
 int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
-                  size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream, float* dobj) {
+                  size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream, float* dobj, float* drel) {
   const int n = g->n_nodes, E = g->n_edges;
   const float inv_keep = dropout_rate > 0.f ? 1.f / (1.f - dropout_rate) : 1.f;
   const Layout L = make_layout(n, E, 1);
@@ -1264,6 +1266,14 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
         SPW_KLAUNCH("k_edge_step_bwd", kw, dim3(egrid), dim3(kThreads), edge_bwd_smem(), st, a);
       }
 #endif
+      if (drel) {   // this step's term of d drel, before the next step overwrites DH1 and dH2S
+        RelGradStepArgs r;
+        r.E = E; r.in_snd = g->in_snd; r.in_rcv = g->in_rcv; r.DH1 = ws + L.DH1; r.A = ws + L.A; r.e_ld = kDEP;
+        r.S = l > 0 ? S : nullptr; r.R = l > 0 ? R : nullptr; r.s_ld = kDEP; r.dH2S = ws + L.dH2S; r.h_ld = kDEP;
+        r.bits_h2 = reinterpret_cast<const uint8_t*>(a.maskbits); r.bits_rows = 0; r.dG = dG; r.g_ld = kDP;
+        r.b2 = w->rmp_b[1]; r.b3 = w->rmp_b[2]; r.first = a.first; r.drel = drel;
+        SPW_KLAUNCH_PDL("k_rel_grad_step", k_rel_grad_step<false>, dim3(grid_for(E, 256)), dim3(256), 0, st, r);
+      }
     }
     if (l > 0) {
       float* dS = ws + L.dS + (size_t)(l - 1) * nE;
@@ -1355,7 +1365,7 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
     a.RM1 = PK(P_RM1); a.RM2 = PK(P_RM2); a.RM3 = PK(P_RM3); a.b1 = w->rm_b[1]; a.b2 = w->rm_b[2]; a.b3 = w->rm_b[3];
     a.RM1T = PK(P_RM1T); a.RM2T = PK(P_RM2T); a.RM3T = PK(P_RM3T); a.W1AT = PK(P_W1AT); a.dA = ws + L.dA;
     a.X1 = ws + L.EX1; a.X2 = ws + L.EX2; a.C = ws + L.EC; a.inv_keep = inv_keep;
-    a.partM = ws + L.partM; a.part0 = ws + L.part0; a.G0 = dobj ? ws + L.GB : nullptr;
+    a.partM = ws + L.partM; a.part0 = ws + L.part0; a.G0 = dobj || drel ? ws + L.GB : nullptr;
     set_smem(k_edge_encode_bwd, edge_encb_smem());
     SPW_KLAUNCH("k_edge_encode_bwd", k_edge_encode_bwd, dim3(bgrid), dim3(kThreads), edge_encb_smem(), st, a);
     if (grads) {
@@ -1385,7 +1395,13 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
     a.rm_w0 = w->rm_w[0]; a.om_w0 = w->om_w[0]; a.dobj = dobj;
     SPW_KLAUNCH_PDL("k_obj_grad_c", k_obj_grad_c<false>, dim3(grid_for(n, 256)), dim3(256), 0, st, a);
   }
-  return check_launch(grads ? "spw_backward" : "spw_backward_obj");
+  if (drel && E > 0) {   // the encoder term of d drel from D_e (in GB)
+    RelGradEncArgs a;
+    a.E = E; a.in_snd = g->in_snd; a.in_rcv = g->in_rcv; a.obj = obj; a.G0 = ws + L.GB; a.g_ld = kDEP;
+    a.rm_w0 = w->rm_w[0]; a.drel = drel;
+    SPW_KLAUNCH_PDL("k_rel_grad_enc", k_rel_grad_enc<false>, dim3(grid_for(E, 256)), dim3(256), 0, st, a);
+  }
+  return check_launch(grads ? "spw_backward" : drel ? "spw_backward_rel" : "spw_backward_obj");
 }
 }  // namespace
 
@@ -1405,7 +1421,7 @@ int spw_backward(const SpwParams* w, const SpwGraph* g, const float* obj, const 
     return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, grads, dropout_rate, (cudaStream_t)stream);
   }
 #endif
-  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, grads, dropout_rate, stream, nullptr);
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, grads, dropout_rate, stream, nullptr, nullptr);
 }
 
 int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
@@ -1422,7 +1438,28 @@ int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, co
   if (!use_csl()) return fail(SPW_ERR_UNSUPPORTED, "spw_backward_obj: not implemented on the round-1 data path (SPW_CSL=0)");
   return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, nullptr, dropout_rate, (cudaStream_t)stream, dobj);
 #else
-  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj);
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj, nullptr);
+#endif
+}
+
+int spw_backward_rel(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
+                     size_t workspace_bytes, float dropout_rate, float* drel, float* dobj, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_backward_rel")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (g->n_nodes == 0) return SPW_OK;
+  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward_rel: workspace null or not 16-byte aligned");
+  if (!obj || !dlogits || (!drel && g->n_edges > 0)) return fail(SPW_ERR_BAD_ARG, "spw_backward_rel: null pointer");
+  if (reinterpret_cast<uintptr_t>(drel) % sizeof(float)) return fail(SPW_ERR_BAD_ARG, "spw_backward_rel: drel not 4-byte aligned");
+  if (dobj && !aligned16(dobj)) return fail(SPW_ERR_BAD_ARG, "spw_backward_rel: dobj not 16-byte aligned");
+  if (dropout_rate < 0.f || dropout_rate >= 1.f) return fail(SPW_ERR_BAD_ARG, "spw_backward_rel: dropout rate %g outside [0,1)", dropout_rate);
+  if (g->n_edges == 0 && !dobj) return SPW_OK;
+  float* dr = g->n_edges > 0 ? drel : nullptr;
+#if SPW_USE_TC
+  if (!use_csl()) return fail(SPW_ERR_UNSUPPORTED, "spw_backward_rel: not implemented on the round-1 data path (SPW_CSL=0)");
+  return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, nullptr, dropout_rate, (cudaStream_t)stream, dobj, dr);
+#else
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj, dr);
 #endif
 }
 

@@ -171,6 +171,27 @@ class Engine:
                                            _stream_ptr(self.device)))
         return self.grads
 
+    def relation_gradients(self, batch, dlogits):
+        """Gradient of sum(dlogits*logits) with respect to the relation weights and the block features, from one pass of
+        spw_backward_rel: (drel (n_edges,), dobj (n_nodes, 3)), fp32 on the device.  drel[k] belongs to the receiver-major
+        relation batch.in_snd[k] -> batch.in_rcv[k] (include/spwgnn.h says how to reach the slot order); dobj equals
+        PropNetObjFunction's gradient bit for bit.  dlogits: (n_nodes,) tensor, or a function of the forward's fp32 logits that
+        returns one (for a seed such as p (1 - p)).  The forward pass is PropNetObjFunction's (a training forward at dropout
+        rate 0 into a workspace owned by this call), so a training step in flight on this Engine is left alone."""
+        api, n, E = self.api, batch.n_nodes, batch.n_edges
+        logits, ws, nbytes = _gradient_forward(self, batch, batch.obj.contiguous())
+        dl = (dlogits(logits) if callable(dlogits) else dlogits).detach().to(torch.float32).contiguous()
+        if dl.shape != (n,) or dl.device != self.device:
+            raise SpwError('relation_gradients: dlogits must be (%d,) on %s, got %s on %s' % (n, self.device, tuple(dl.shape), dl.device))
+        with torch.cuda.device(self.device):
+            drel = torch.empty(E, dtype=torch.float32, device=self.device)
+            dobj = torch.empty(n, 3, dtype=torch.float32, device=self.device)
+            wp = self.params.c_struct()
+            api.check(api.dll.spw_backward_rel(ctypes.byref(wp), ctypes.byref(batch.c_graph), batch.obj.data_ptr(), dl.data_ptr(),
+                                               ws.data_ptr(), nbytes, 0.0, drel.data_ptr() if E else None, dobj.data_ptr(),
+                                               _stream_ptr(self.device)))
+        return drel, dobj
+
     def saved_relu_states(self):
         """The relu states the last training forward left for the backward pass, in the oracle's order of relu layers
         (Networks.py:75-76, then :84-90 per step): a list of 21 bool tensors -- rm layers 0..3 [E][150], om layers 0..1
@@ -234,6 +255,20 @@ class PropNetFunction(torch.autograd.Function):
         return g.flat.clone(), None, None
 
 
+def _gradient_forward(engine, batch, obj):
+    """The forward pass of the input gradients: a training spw_forward at dropout rate 0 of `batch` with features `obj` (n, 3)
+    (contiguous fp32 on the engine's device), into a workspace of its own.  Returns (logits, workspace, its size in bytes)."""
+    api, n = engine.api, batch.n_nodes
+    with torch.cuda.device(engine.device):
+        logits = torch.empty(n, dtype=torch.float32, device=engine.device)
+        nbytes = api.dll.spw_workspace_bytes(n, batch.n_edges, 1)
+        ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=engine.device)
+        wp = engine.params.c_struct()
+        api.check(api.dll.spw_forward(ctypes.byref(wp), ctypes.byref(batch.c_graph), obj.data_ptr(), logits.data_ptr(), None,
+                                      ws.data_ptr(), nbytes, 1, 0.0, 0, _stream_ptr(engine.device)))
+    return logits, ws, nbytes
+
+
 class PropNetObjFunction(torch.autograd.Function):
     """torch.autograd bridge for the gradient with respect to the block features: logits = PropNetObjFunction.apply(obj,
     engine, batch).  obj: (n, 3) fp32 on the engine's device, [x, y, width] / 170, used in place of batch.obj; the relations
@@ -250,15 +285,8 @@ class PropNetObjFunction(torch.autograd.Function):
         if obj.shape != (n, 3) or obj.dtype != torch.float32 or obj.device != engine.device:
             raise SpwError('PropNetObjFunction: obj must be (%d, 3) float32 on %s, got %s %s on %s'
                            % (n, engine.device, tuple(obj.shape), obj.dtype, obj.device))
-        api = engine.api
         obj = obj.detach().contiguous()
-        with torch.cuda.device(engine.device):
-            logits = torch.empty(n, dtype=torch.float32, device=engine.device)
-            nbytes = api.dll.spw_workspace_bytes(n, batch.n_edges, 1)
-            ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=engine.device)
-            wp = engine.params.c_struct()
-            api.check(api.dll.spw_forward(ctypes.byref(wp), ctypes.byref(batch.c_graph), obj.data_ptr(), logits.data_ptr(), None,
-                                          ws.data_ptr(), nbytes, 1, 0.0, 0, _stream_ptr(engine.device)))
+        logits, ws, nbytes = _gradient_forward(engine, batch, obj)
         ctx.engine, ctx.batch, ctx.obj, ctx.ws, ctx.nbytes = engine, batch, obj, ws, nbytes
         return logits
 
