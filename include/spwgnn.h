@@ -243,6 +243,27 @@ int spw_backward_obj(const SpwParams* w, const SpwGraph* g, const float* obj, co
 int spw_backward_rel(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
                      size_t workspace_bytes, float dropout_rate, float* drel, float* dobj, void* stream);
 
+/* Gradient of sum_i dlogits[i]*logit[i] with respect to every input of the reference's model (Networks.py:22-99), from one
+ * backward pass without weight gradients: the dense relation tensors sender_relations / receiver_relations (B, N, R) and the
+ * propagation input (B, N, 100), at the relations of g and propagation = 0, and the objects.
+ *   drs, drr [n_edges][max_nodes_per_tower] (4-byte aligned): row k belongs to the receiver-major relation in_snd[k] -> in_rcv[k]
+ *     (its reference slot: see spw_backward_rel), column j to local block j of its tower: d/dsender_relations[j, slot] and
+ *     d/dreceiver_relations[j, slot].  Entries j >= N_t are written as 0.
+ *   drr_free [n_nodes] (4-byte aligned): d/dreceiver_relations[j, slot] of block j at every inactive (all-zero) slot of its tower,
+ *     the same value for all of them (the column's message, that of a zero input, would be delivered to j); d/dsender_relations
+ *     is 0 there.  The message is taken without dropout.
+ *   dprop [n_nodes][100] (16-byte aligned): d/dpropagation.
+ *   dobj: NULL, or [n_nodes][3] (16-byte aligned) receiving spw_backward_obj's result bit for bit.
+ * max_nodes_per_tower: the largest N_t of g (<= SPW_MAX_NODES); a larger tower gets NaN in its rows of drs, drr and drr_free.
+ * workspace / dropout_rate: as spw_backward_obj; the forward state in it is left unchanged.  scratch: at least
+ * spw_backward_inputs_bytes(n_nodes, n_edges) bytes, 16-byte aligned.  All outputs are written, not accumulated.
+ * Deterministic: every sum runs in a fixed order that depends on the tower alone.  n_nodes == 0 launches nothing; with
+ * n_edges == 0, drs and drr may be NULL.  SPW_ERR_UNSUPPORTED on the round-1 data path (SPW_CSL=0). */
+size_t spw_backward_inputs_bytes(int32_t n_nodes, int32_t n_edges);
+int spw_backward_inputs(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj, const float* dlogits,
+                        void* workspace, size_t workspace_bytes, float dropout_rate, void* scratch, size_t scratch_bytes,
+                        float* drs, float* drr, float* drr_free, float* dprop, float* dobj, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -14,7 +14,8 @@ kernels in libspwgnn.so.  Differences by design:
   * `PropagationNetwork(small_batches=True)` sends inference on small batches of small towers through
     `Engine.forward_towers` (one CTA per tower, one launch) instead of the tiled `Engine.forward`;
   * `stability_gradients` differentiates each tower's demolish score with respect to its block poses, and
-    `relation_gradients` with respect to the weights of its relations (which contacts hold the tower up).
+    `relation_gradients` with respect to the weights of its relations (which contacts hold the tower up);
+  * `input_gradients` differentiates predict with respect to all four inputs of the reference's dict (K.gradients).
 """
 import os
 import sys
@@ -260,6 +261,44 @@ class PropagationModel:
         eo = batch.out_off[:batch.n_nodes + 1].cpu().numpy().astype(np.int64)[off]
         return [(np.stack([snd[eo[t]:eo[t + 1]], rcv[eo[t]:eo[t + 1]]], 1) - off[t], val[eo[t]:eo[t + 1]])
                 for t in range(batch.n_towers)]
+
+    def input_gradients(self, x, dprobs=None):
+        """The gradient of sum(dprobs * p) with respect to the four inputs of the reference's model, p = predict(x): what
+        K.gradients(model.output, model.inputs, grad_ys=dprobs) returns for the reference's Keras model (Networks.py:22-99).
+        x: the reference's dict; dprobs: (B, N, 1) or (B, N), default ones.  Returns a dict with the keys and shapes of x
+        ('objects' (B, N, 3), 'sender_relations' / 'receiver_relations' (B, N, R), 'propagation' (B, N, 100)), float32: the
+        gradients at every entry of the relation tensors, zero and inactive ones included, and at propagation = 0 (the forward
+        implies that seed, so a nonzero 'propagation' raises).  One packed pass of Engine.input_gradients with the seed
+        dprobs * p (1 - p), p = sigmoid(logits) in fp32."""
+        obj = np.asarray(x['objects'])
+        B, N = obj.shape[:2]
+        R = np.asarray(x['sender_relations']).shape[2]
+        if x.get('propagation') is not None and np.any(np.asarray(x['propagation']) != 0):
+            raise SpwError('input_gradients: the forward pass implies propagation = 0; a nonzero propagation input is not supported')
+        eng = self.engine
+        if dprobs is None:
+            dp = torch.ones(B * N, dtype=torch.float32, device=eng.device)
+        else:
+            dp = torch.as_tensor(np.asarray(dprobs, dtype=np.float32))
+            if tuple(dp.shape) not in ((B, N, 1), (B, N)):
+                raise SpwError('input_gradients: dprobs must be (%d, %d, 1) or (%d, %d), got %s' % (B, N, B, N, tuple(dp.shape)))
+            dp = dp.reshape(B * N).to(eng.device)
+        batch = self._batch_from_dict(x)
+
+        def seed(z):
+            p = torch.sigmoid(z)
+            return dp * (p * (1 - p))
+        drs, drr, free, dprop, dobj = eng.input_gradients(batch, seed)
+        d_rs = torch.zeros(B, N, R, dtype=torch.float32, device=eng.device)
+        d_rr = free.reshape(B, N, 1).expand(B, N, R).contiguous()        # inactive slots: 0 and drr_free
+        E = batch.n_edges
+        if E:
+            snd, _, slot = batch.slot_list                                  # slot (sender-major) order
+            o, b, sl = batch.out_pos[:E].long(), snd[:E].long() // N, slot[:E].long()
+            d_rs[b, :, sl] = drs[o, :N]
+            d_rr[b, :, sl] = drr[o, :N]
+        return {'objects': dobj.reshape(B, N, 3).cpu().numpy(), 'sender_relations': d_rs.cpu().numpy(),
+                'receiver_relations': d_rr.cpu().numpy(), 'propagation': dprop.reshape(B, N, 100).cpu().numpy()}
 
     # ---- training ------------------------------------------------------------------------------
     def train_on_batch(self, batch, target):

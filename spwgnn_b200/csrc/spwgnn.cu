@@ -13,6 +13,7 @@
 #include "spw_small.cuh"
 #include "spw_obj_grad.cuh"
 #include "spw_rel_grad.cuh"
+#include "spw_input_grad.cuh"
 
 #include <stdarg.h>
 #include <stdio.h>
@@ -1167,9 +1168,12 @@ int spw_bce_grad(const float* logits, const float* target, int32_t n_nodes, doub
 namespace {
 // The backward pass of the row-major data path (round 1; the only one of the FFMA build).  grads == null (spw_backward_obj):
 // no weight gradient is reduced; dobj != null: d obj [n][3] from the layer-0 gradients (k_obj_grad_c, spw_obj_grad.cuh);
-// drel != null: d drel [E] with respect to the relation weights (k_rel_grad_step / k_rel_grad_enc, spw_rel_grad.cuh).
+// drel != null: d drel [E] with respect to the relation weights (k_rel_grad_step / k_rel_grad_enc, spw_rel_grad.cuh);
+// ig != null: the gradients with respect to the dense relation tensors and the propagation input (spw_input_grad.cuh; dS / dR
+// slot 0 take step 0's sender / receiver sums, and d prop is formed in place).
 int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const float* dlogits, void* workspace,
-                  size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream, float* dobj, float* drel) {
+                  size_t workspace_bytes, const SpwParams* grads, float dropout_rate, void* stream, float* dobj, float* drel,
+                  const InputGradTarget* ig = nullptr) {
   const int n = g->n_nodes, E = g->n_edges;
   const float inv_keep = dropout_rate > 0.f ? 1.f / (1.f - dropout_rate) : 1.f;
   const Layout L = make_layout(n, E, 1);
@@ -1197,6 +1201,13 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
   float* dU5 = ws + L.dU + 4 * nP;
   const float* U5 = ws + L.U + 4 * nP;
   SPW_KLAUNCH("k_logit_bwd", k_logit_bwd, dim3(grid_for((int64_t)n * kDP, 256)), dim3(256), 0, st, dlogits, U5, n, w->omp_w[1], dU5);
+  const InputGradScratch IS = input_grad_scratch(n, E);
+  if (ig) {   // h2_0: the hidden state of the message of an all-zero relation column
+    ZeroMessageArgs z;
+    for (int i = 0; i < 4; ++i) { z.rm_w[i] = w->rm_w[i]; z.rm_b[i] = w->rm_b[i]; }
+    z.w1a = w->rmp_w[0]; z.b1 = w->rmp_b[0]; z.w2 = w->rmp_w[1]; z.b2 = w->rmp_b[1]; z.h2_0 = ig->scratch + IS.H20;
+    SPW_KLAUNCH_PDL("k_zero_message", k_zero_message, dim3(1), dim3(256), 0, st, z);
+  }
 
   for (int l = SPW_N_STEPS - 1; l >= 0; --l) {   // step l+1 of the forward loop
     const float* Pin = ws + L.P + (size_t)l * nP;
@@ -1222,10 +1233,10 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
       LinOpt o; o.mulsrc = G; o.ld_mul = kDP; o.mulmode = 2;
       run_linear(st, ws, L, {T_V1BT, P_V1BT, 0}, n, kDP, 1, &s, dG, kDP, o);
     }
-    if (l > 0) {   // DP = dUpre.V1c^T (+ residual T)
+    if (l > 0 || ig) {   // DP = dUpre.V1c^T (+ residual T); step 0: the first term of d prop, in place
       RowsSeg s = {dU, kDP, kDP};
       LinOpt o; o.addend = Tl; o.ld_add = kDP;
-      run_linear(st, ws, L, {T_V1CT, P_V1CT, 0}, n, kDP, 1, &s, ws + L.DP, kDP, o);
+      run_linear(st, ws, L, {T_V1CT, P_V1CT, 0}, n, kDP, 1, &s, l > 0 ? ws + L.DP : ig->dprop, kDP, o);
     }
     {   // d(sum h2) = dg_pre.W3^T
       RowsSeg s = {dG, kDP, kDP};
@@ -1275,9 +1286,26 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
         SPW_KLAUNCH_PDL("k_rel_grad_step", k_rel_grad_step<false>, dim3(grid_for(E, 256)), dim3(256), 0, st, r);
       }
     }
-    if (l > 0) {
-      float* dS = ws + L.dS + (size_t)(l - 1) * nE;
-      float* dR = ws + L.dR + (size_t)(l - 1) * nE;
+    if (ig) {   // this step's terms of d Rs, d Rr and of the inactive slots, before the next step overwrites DH1 and dH2S
+      float* H2 = ig->scratch + IS.H2;
+      if (E > 0) {
+        H2RowsArgs h;
+        h.E = E; h.in_snd = g->in_snd; h.in_rcv = g->in_rcv; h.A = ws + L.A; h.S = l > 0 ? S : nullptr; h.R = l > 0 ? R : nullptr;
+        h.bits_h2 = reinterpret_cast<const uint32_t*>(ws + L.M2) + (size_t)l * E * 8; h.w2 = w->rmp_w[1]; h.b2 = w->rmp_b[1]; h.H2 = H2;
+        SPW_KLAUNCH_PDL("k_h2_rows", k_h2_rows, dim3(grid_for((int64_t)E * kDEP, 256)), dim3(256), 0, st, h);
+      }
+      InputGradStepArgs a;
+      a.T = g->n_towers; a.node_off = g->node_off; a.in_off = g->in_off; a.max_nodes = ig->max_nodes;
+      a.DH1 = ws + L.DH1; a.H2 = H2; a.e_ld = kDEP; a.S = l > 0 ? S : nullptr; a.R = l > 0 ? R : nullptr; a.s_ld = kDEP;
+      a.dH2S = ws + L.dH2S; a.h_ld = kDEP; a.dG = dG; a.g_ld = kDP; a.b3 = w->rmp_b[2]; a.h2_0 = ig->scratch + IS.H20;
+      a.first = l == SPW_N_STEPS - 1; a.drs = ig->drs; a.drr = ig->drr; a.drr_free = ig->drr_free;
+      const size_t sm = input_grad_step_smem(ig->max_nodes);
+      set_smem(k_input_grad_step<false>, sm);
+      SPW_KLAUNCH_PDL("k_input_grad_step", k_input_grad_step<false>, dim3(g->n_towers), dim3(256), sm, st, a);
+    }
+    if (l > 0 || ig) {
+      float* dS = ws + L.dS + (size_t)(l > 0 ? l - 1 : 0) * nE;
+      float* dR = ws + L.dR + (size_t)(l > 0 ? l - 1 : 0) * nE;
       if (E > 0) {
         SPW_KLAUNCH("k_gather_dsr", k_gather_dsr, dim3(grid_for(n, 8)), dim3(256), 0, st, n, g->in_off, g->out_off, g->out_pos,
                    ws + L.DH1, dS, dR);
@@ -1289,6 +1317,11 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
       //   two K = 150 products: the first one is added into DP, the second one finishes T
       RowsSeg s1 = {dS, kDEP, kDE}, s2 = {dR, kDEP, kDE};
       LinOpt o1; o1.accumulate = 1;
+      if (l == 0) {   // d prop += dS^0.W1b^T + dR^0.W1c^T: the l > 0 expression below where 1 - (p^0)^2 = 1
+        run_linear(st, ws, L, {T_W1BT, P_W1BT, 0}, n, kDP, 1, &s1, ig->dprop, kDP, o1);
+        run_linear(st, ws, L, {T_W1CT, P_W1CT, 0}, n, kDP, 1, &s2, ig->dprop, kDP, o1);
+        continue;
+      }
       run_linear(st, ws, L, {T_W1BT, P_W1BT, 0}, n, kDP, 1, &s1, ws + L.DP, kDP, o1);
       LinOpt o; o.addend = ws + L.DP; o.ld_add = kDP; o.mulsrc = Pin; o.ld_mul = kDP; o.mulmode = 2;
       run_linear(st, ws, L, {T_W1CT, P_W1CT, 0}, n, kDP, 1, &s2, ws + L.T + (size_t)(l - 1) * nP, kDP, o);
@@ -1365,7 +1398,7 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
     a.RM1 = PK(P_RM1); a.RM2 = PK(P_RM2); a.RM3 = PK(P_RM3); a.b1 = w->rm_b[1]; a.b2 = w->rm_b[2]; a.b3 = w->rm_b[3];
     a.RM1T = PK(P_RM1T); a.RM2T = PK(P_RM2T); a.RM3T = PK(P_RM3T); a.W1AT = PK(P_W1AT); a.dA = ws + L.dA;
     a.X1 = ws + L.EX1; a.X2 = ws + L.EX2; a.C = ws + L.EC; a.inv_keep = inv_keep;
-    a.partM = ws + L.partM; a.part0 = ws + L.part0; a.G0 = dobj || drel ? ws + L.GB : nullptr;
+    a.partM = ws + L.partM; a.part0 = ws + L.part0; a.G0 = dobj || drel || ig ? ws + L.GB : nullptr;
     set_smem(k_edge_encode_bwd, edge_encb_smem());
     SPW_KLAUNCH("k_edge_encode_bwd", k_edge_encode_bwd, dim3(bgrid), dim3(kThreads), edge_encb_smem(), st, a);
     if (grads) {
@@ -1401,7 +1434,13 @@ int backward_rows(const SpwParams* w, const SpwGraph* g, const float* obj, const
     a.rm_w0 = w->rm_w[0]; a.drel = drel;
     SPW_KLAUNCH_PDL("k_rel_grad_enc", k_rel_grad_enc<false>, dim3(grid_for(E, 256)), dim3(256), 0, st, a);
   }
-  return check_launch(grads ? "spw_backward" : drel ? "spw_backward_rel" : "spw_backward_obj");
+  if (ig && E > 0) {   // the encoder term of d Rs / d Rr from D_e (in GB)
+    InputGradEncArgs a;
+    a.T = g->n_towers; a.node_off = g->node_off; a.in_off = g->in_off; a.max_nodes = ig->max_nodes; a.obj = obj;
+    a.G0 = ws + L.GB; a.g_ld = kDEP; a.rm_w0 = w->rm_w[0]; a.drs = ig->drs; a.drr = ig->drr;
+    SPW_KLAUNCH_PDL("k_input_grad_enc", k_input_grad_enc<false>, dim3(g->n_towers), dim3(256), 0, st, a);
+  }
+  return check_launch(grads ? "spw_backward" : drel ? "spw_backward_rel" : ig ? "spw_backward_inputs" : "spw_backward_obj");
 }
 }  // namespace
 
@@ -1460,6 +1499,44 @@ int spw_backward_rel(const SpwParams* w, const SpwGraph* g, const float* obj, co
   return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, nullptr, dropout_rate, (cudaStream_t)stream, dobj, dr);
 #else
   return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj, dr);
+#endif
+}
+
+size_t spw_backward_inputs_bytes(int32_t n_nodes, int32_t n_edges) {
+  if (n_nodes < 0 || n_edges < 0) return 0;
+  return input_grad_scratch(n_nodes, n_edges).total * sizeof(float);
+}
+
+int spw_backward_inputs(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj, const float* dlogits,
+                        void* workspace, size_t workspace_bytes, float dropout_rate, void* scratch, size_t scratch_bytes, float* drs,
+                        float* drr, float* drr_free, float* dprop, float* dobj, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_backward_inputs")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (max_nodes_per_tower < 0 || max_nodes_per_tower > SPW_MAX_NODES)
+    return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: max_nodes_per_tower %d outside [0, %d]", max_nodes_per_tower, SPW_MAX_NODES);
+  if (g->n_nodes == 0) return SPW_OK;
+  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: workspace null or not 16-byte aligned");
+  if (!scratch || !aligned16(scratch)) return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: scratch null or not 16-byte aligned");
+  if (!obj || !dlogits || !drr_free || !dprop || ((!drs || !drr) && g->n_edges > 0))
+    return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: null pointer");
+  if (reinterpret_cast<uintptr_t>(drs) % sizeof(float) || reinterpret_cast<uintptr_t>(drr) % sizeof(float) ||
+      reinterpret_cast<uintptr_t>(drr_free) % sizeof(float))
+    return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: drs, drr or drr_free not 4-byte aligned");
+  if (!aligned16(dprop)) return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: dprop not 16-byte aligned");
+  if (dobj && !aligned16(dobj)) return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: dobj not 16-byte aligned");
+  if (dropout_rate < 0.f || dropout_rate >= 1.f) return fail(SPW_ERR_BAD_ARG, "spw_backward_inputs: dropout rate %g outside [0,1)", dropout_rate);
+  const size_t need = spw_backward_inputs_bytes(g->n_nodes, g->n_edges);
+  if (scratch_bytes < need) return fail(SPW_ERR_WORKSPACE, "spw_backward_inputs: scratch %zu < %zu bytes", scratch_bytes, need);
+  InputGradTarget t;
+  t.max_nodes = max_nodes_per_tower; t.scratch = reinterpret_cast<float*>(scratch);
+  t.drs = drs; t.drr = drr; t.drr_free = drr_free; t.dprop = dprop;
+#if SPW_USE_TC
+  if (!use_csl()) return fail(SPW_ERR_UNSUPPORTED, "spw_backward_inputs: not implemented on the round-1 data path (SPW_CSL=0)");
+  return backward_csl(w, g, obj, dlogits, reinterpret_cast<float*>(workspace), workspace_bytes, nullptr, dropout_rate, (cudaStream_t)stream, dobj,
+                      nullptr, &t);
+#else
+  return backward_rows(w, g, obj, dlogits, workspace, workspace_bytes, nullptr, dropout_rate, stream, dobj, nullptr, &t);
 #endif
 }
 

@@ -192,6 +192,32 @@ class Engine:
                                                _stream_ptr(self.device)))
         return drel, dobj
 
+    def input_gradients(self, batch, dlogits):
+        """Gradient of sum(dlogits*logits) with respect to every input of the reference's model, from one pass of
+        spw_backward_inputs: (drs, drr (n_edges, batch.max_nodes), drr_free (n_nodes,), dprop (n_nodes, 100), dobj (n_nodes, 3)),
+        fp32 on the device.  Row k of drs / drr is the sender_relations / receiver_relations column of the receiver-major
+        relation batch.in_snd[k] -> batch.in_rcv[k], entry j local block j of its tower (0 past the tower's size); drr_free[i]
+        is d/dreceiver_relations at every inactive slot of block i's tower; dprop is d/dpropagation at 0; dobj equals
+        PropNetObjFunction's gradient bit for bit (include/spwgnn.h).  dlogits: (n_nodes,) tensor, or a function of the
+        forward's fp32 logits that returns one.  The forward pass is PropNetObjFunction's (a training forward at dropout rate 0
+        into a workspace owned by this call), so a training step in flight on this Engine is left alone."""
+        api, n, E, mx = self.api, batch.n_nodes, batch.n_edges, batch.max_nodes
+        logits, ws, nbytes = _gradient_forward(self, batch, batch.obj.contiguous())
+        dl = (dlogits(logits) if callable(dlogits) else dlogits).detach().to(torch.float32).contiguous()
+        if dl.shape != (n,) or dl.device != self.device:
+            raise SpwError('input_gradients: dlogits must be (%d,) on %s, got %s on %s' % (n, self.device, tuple(dl.shape), dl.device))
+        with torch.cuda.device(self.device):
+            new = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=self.device)
+            drs, drr, free, dprop, dobj = new(E, mx), new(E, mx), new(n), new(n, 100), new(n, 3)
+            sb = api.dll.spw_backward_inputs_bytes(n, E)
+            scratch = torch.empty(max(sb, 1), dtype=torch.uint8, device=self.device)
+            wp = self.params.c_struct()
+            api.check(api.dll.spw_backward_inputs(ctypes.byref(wp), ctypes.byref(batch.c_graph), mx, batch.obj.data_ptr(), dl.data_ptr(),
+                                                  ws.data_ptr(), nbytes, 0.0, scratch.data_ptr(), sb,
+                                                  drs.data_ptr() if E else None, drr.data_ptr() if E else None, free.data_ptr(),
+                                                  dprop.data_ptr(), dobj.data_ptr(), _stream_ptr(self.device)))
+        return drs, drr, free, dprop, dobj
+
     def saved_relu_states(self):
         """The relu states the last training forward left for the backward pass, in the oracle's order of relu layers
         (Networks.py:75-76, then :84-90 per step): a list of 21 bool tensors -- rm layers 0..3 [E][150], om layers 0..1
