@@ -208,6 +208,26 @@ size_t spw_forward_towers_bytes(int32_t n_nodes, int32_t n_edges);
 int spw_forward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj, float* logits,
                        float* probs, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The backward pass of spw_forward_towers, in ONE launch with one CTA per tower: each tower's logits and the gradients of
+ * sum_i (dlogits[i] logit_i + dprobs[i] p_i) with respect to the block features and, optionally, the relation weights,
+ * p = sigmoid(logit).  The forward pass is spw_forward_towers' code, so the logits are its bits; every sum runs in a fixed
+ * order that depends on the tower alone, so a tower's logits, dobj and drel are the same bits whatever else is in the
+ * batch and wherever it sits in it.  Plain fp32 FFMA, no dropout.
+ *   max_nodes_per_tower: as spw_forward_towers; a tower with more blocks gets NaN logits, dobj rows and drel of its
+ *                        relations, and nothing else of it is written.
+ *   dlogits, dprobs [n_nodes]: the seed dlogit_i = dlogits[i] + dprobs[i] p_i (1 - p_i); either may be NULL (read as 0),
+ *                              not both.
+ *   logits: NULL or [n_nodes], written with spw_forward_towers' values.
+ *   dobj [n_nodes][3], 16-byte aligned: as spw_backward_obj.
+ *   drel: NULL or [n_edges] in the receiver-major relation order, as spw_backward_rel; may be NULL when n_edges == 0.
+ *   workspace: at least spw_backward_towers_bytes(n_nodes, n_edges) bytes, 16-byte aligned.  Nothing in it is kept after
+ *              the call.
+ * n_nodes == 0 launches nothing. */
+size_t spw_backward_towers_bytes(int32_t n_nodes, int32_t n_edges);
+int spw_backward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj,
+                        const float* dlogits, const float* dprobs, float* logits, float* dobj, float* drel,
+                        void* workspace, size_t workspace_bytes, void* stream);
+
 /* Keras binary_crossentropy on probabilities clipped to [1e-7, 1-1e-7] (Networks.py:102), mean over
  * `count` outputs (pass the GLOBAL number of blocks when data-parallel).  Writes dlogits [n_nodes]
  * = d(mean loss)/d(logit) and adds the summed loss and the number of correct (p>0.5)==target

@@ -57,9 +57,12 @@ class PropagationNetwork:
     small_batches=True: every inference call of the models (predict, predict_logits, predict_towers, predict_tower_sums,
     score_removals, score_drops, evaluate and the validation pass of fit / fit_towers) uses Engine.forward_towers when the
     batch's towers have at most `small_max_nodes` blocks and there are at most `small_max_towers` of them, and the tiled
-    Engine.forward otherwise.  Training is unchanged.  On that path a tower's probabilities do not depend on the rest of the
-    batch, bit for bit: a packed demolish search (score_removals, score_drops) gives exactly the sums of one batch-1 predict
-    per candidate.  Off by default: the two paths agree to fp32 rounding, not bit for bit, and the tiled path is faster."""
+    Engine.forward otherwise; stability_gradients and relation_gradients use Engine.gradients_towers (the backward pass of
+    the same kernel's forward, one launch) under the same limits, so predictions and their gradients come from one fp32
+    function.  Training and input_gradients are unchanged.  On that path a tower's probabilities and gradients do not depend
+    on the rest of the batch, bit for bit: a packed demolish search (score_removals, score_drops) gives exactly the sums of
+    one batch-1 predict per candidate, and a packed stability_gradients call the gradients of one batch-1 call per tower.
+    Off by default: the two paths agree to fp32 rounding, not bit for bit, and the tiled path is faster."""
 
     # The limits keep forward_towers where its cost stays within about 2x of the tiled path.  It wins nowhere yet: measured
     # on one B200 at a 1000 W power limit (tools/bench_small.py, profiles/small_r05.json), device time per call, tiled vs
@@ -116,11 +119,16 @@ class PropagationModel:
         return self.network.engine
 
     # ---- inference -----------------------------------------------------------------------------
+    def _small(self, batch):
+        """True when the batch takes the per-tower kernels: small_batches=True and the batch inside the network's limits."""
+        net = self.network
+        return net.small_batches and batch.max_nodes <= net.small_max_nodes and batch.n_towers <= net.small_max_towers
+
     def _infer(self, batch, want_probs=True):
         """The inference forward of every call below: forward_towers for small batches of small towers when the network
         was built with small_batches=True, the tiled forward otherwise."""
-        net, eng = self.network, self.engine
-        if net.small_batches and batch.max_nodes <= net.small_max_nodes and batch.n_towers <= net.small_max_towers:
+        eng = self.engine
+        if self._small(batch):
             return eng.forward_towers(batch, want_probs=want_probs)
         return eng.forward(batch, training=False, want_probs=want_probs)
 
@@ -218,17 +226,22 @@ class PropagationModel:
         [x, y, width]: a list of (N_t, 3) float64 arrays, in pixels.  `towers` and the relation options are those of
         predict_towers; the relations are held fixed (they come from a distance threshold, which is piecewise constant).
         Towers are independent, so one packed backward pass of the batch's total gives every tower the gradient of its own
-        sum.  p = sigmoid(logits) in fp32; the factor 1/170 of the feature normalisation is applied in float64.  Always the
-        tiled path (PropNetObjFunction): the per-tower kernel of small_batches=True has no backward pass."""
+        sum.  p = sigmoid(logits) in fp32; the factor 1/170 of the feature normalisation is applied in float64.  The path is
+        the one predict takes: Engine.gradients_towers (seed dprobs = 1) when _infer would use forward_towers, else the tiled
+        PropNetObjFunction."""
         if not towers:
             return []
         eng = self.engine
         batch = TowerBatch.from_towers(towers, thr=thr, fully_connected=fully_connected, inference_glue=inference_glue,
                                        device=eng.device)
-        obj = batch.obj.detach().clone().requires_grad_(True)
-        with torch.enable_grad():
-            p = torch.sigmoid(PropNetObjFunction.apply(obj, eng, batch))
-            (g,) = torch.autograd.grad(p.sum(), [obj])
+        if self._small(batch):
+            ones = torch.ones(batch.n_nodes, dtype=torch.float32, device=eng.device)
+            _, g, _ = eng.gradients_towers(batch, dprobs=ones)
+        else:
+            obj = batch.obj.detach().clone().requires_grad_(True)
+            with torch.enable_grad():
+                p = torch.sigmoid(PropNetObjFunction.apply(obj, eng, batch))
+                (g,) = torch.autograd.grad(p.sum(), [obj])
         g = g.cpu().numpy().astype(np.float64) / REL_THRESHOLD
         off = batch.node_off_host
         return [g[off[t]:off[t + 1]] for t in range(batch.n_towers)]
@@ -240,7 +253,8 @@ class PropagationModel:
         tower, (pairs, grads): pairs (E_t, 2) int64 local (sender, receiver) block indices of the tower's active relations in
         the reference's slot order (main.py:69-81: sender outer, receiver inner), grads (E_t,) float64.  Weights are
         dimensionless, so no 1/170 factor applies.  `towers` and the relation options are those of predict_towers; one packed
-        pass of Engine.relation_gradients with the seed p (1 - p) serves the whole batch."""
+        pass of Engine.relation_gradients with the seed p (1 - p) serves the whole batch, or of Engine.gradients_towers with
+        dprobs = 1 when _infer would use forward_towers (small_batches=True)."""
         if not towers:
             return []
         eng = self.engine
@@ -250,7 +264,11 @@ class PropagationModel:
         def seed(z):
             p = torch.sigmoid(z)
             return p * (1 - p)
-        drel, _ = eng.relation_gradients(batch, seed)
+        if self._small(batch):
+            ones = torch.ones(batch.n_nodes, dtype=torch.float32, device=eng.device)
+            _, _, drel = eng.gradients_towers(batch, dprobs=ones, want_drel=True)
+        else:
+            drel, _ = eng.relation_gradients(batch, seed)
         E, off = batch.n_edges, batch.node_off_host
         if E == 0:
             return [(np.zeros((0, 2), np.int64), np.zeros(0, np.float64)) for _ in range(batch.n_towers)]

@@ -33,7 +33,7 @@ class SpwGraph(C.Structure):
 
 
 EXPORTS = ['spw_version', 'spw_last_error', 'spw_launch_count', 'spw_profile', 'spw_profile_report', 'spw_ffma_peak', 'spw_tc_selftest', 'spw_tc2_selftest', 'spw_tc_linear', 'spw_csl_linear', 'spw_edges_count', 'spw_edges_fill', 'spw_sample_sizes', 'spw_sample_jenga', 'spw_sample_tower', 'spw_candidates_remove', 'spw_candidates_drop', 'spw_tower_sums', 'spw_workspace_bytes', 'spw_saved_state_layout',
-           'spw_workspace_layout_names', 'spw_workspace_layout', 'spw_forward', 'spw_forward_towers_bytes', 'spw_forward_towers', 'spw_bce_grad', 'spw_backward', 'spw_backward_obj', 'spw_backward_rel',
+           'spw_workspace_layout_names', 'spw_workspace_layout', 'spw_forward', 'spw_forward_towers_bytes', 'spw_forward_towers', 'spw_backward_towers_bytes', 'spw_backward_towers', 'spw_bce_grad', 'spw_backward', 'spw_backward_obj', 'spw_backward_rel',
            'spw_backward_inputs_bytes', 'spw_backward_inputs']
 
 
@@ -103,6 +103,10 @@ class CApi:
         d.spw_forward_towers_bytes.argtypes = [i32, i32]
         d.spw_forward_towers.restype = C.c_int
         d.spw_forward_towers.argtypes = [C.POINTER(SpwParams), C.POINTER(SpwGraph), i32, vp, vp, vp, vp, C.c_size_t, vp]
+        d.spw_backward_towers_bytes.restype = C.c_size_t
+        d.spw_backward_towers_bytes.argtypes = [i32, i32]
+        d.spw_backward_towers.restype = C.c_int
+        d.spw_backward_towers.argtypes = [C.POINTER(SpwParams), C.POINTER(SpwGraph), i32, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
         d.spw_bce_grad.restype = C.c_int
         d.spw_bce_grad.argtypes = [vp, vp, i32, f64, vp, vp, vp]
         d.spw_backward.restype = C.c_int

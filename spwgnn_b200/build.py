@@ -5,7 +5,7 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, 'csrc', 'spwgnn.cu')
-DEPS = [os.path.join(HERE, 'csrc', f) for f in ('spwgnn.cu', 'spw_common.cuh', 'spw_edges.cuh', 'spw_kernels.cuh', 'spw_tc.cuh', 'spw_rows_tc.cuh', 'spw_pipe_tc.cuh', 'spw_csl.cuh', 'spw_csl_kernels.cuh', 'spw_csl_wgrad.cuh', 'spw_csl_path.inl', 'spw_small.cuh', 'spw_obj_grad.cuh', 'spw_rel_grad.cuh', 'spw_input_grad.cuh')] + \
+DEPS = [os.path.join(HERE, 'csrc', f) for f in ('spwgnn.cu', 'spw_common.cuh', 'spw_edges.cuh', 'spw_kernels.cuh', 'spw_tc.cuh', 'spw_rows_tc.cuh', 'spw_pipe_tc.cuh', 'spw_csl.cuh', 'spw_csl_kernels.cuh', 'spw_csl_wgrad.cuh', 'spw_csl_path.inl', 'spw_small.cuh', 'spw_small_grad.cuh', 'spw_obj_grad.cuh', 'spw_rel_grad.cuh', 'spw_input_grad.cuh')] + \
        [os.path.join(os.path.dirname(HERE), 'include', 'spwgnn.h')]
 OUT = os.path.join(HERE, 'libspwgnn.so')
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '--shared',

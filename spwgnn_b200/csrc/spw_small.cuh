@@ -64,26 +64,45 @@ inline size_t small_smem_bytes(int maxn) { return (size_t)small_smem_layout(maxn
 // [lane C, lane C + C).  Each sum is one fmaf chain in increasing k, so the result does not depend on R or on which warp
 // computes the row.  Every thread of the CTA must call it (barriers inside); it ends with a barrier before the epilogue.
 constexpr int kSmallKT = 32;
-template <int C>
+// TRANS = false: tile element (kr, c) is W[(k0 + kr) ldw + c] (the product X.W); TRANS = true: it is W[c ldw + k0 + kr] (the
+// product X.W^T of the backward pass, W still in Keras layout).  The transposed tile is read 8 k-rows x 4 columns per warp
+// (32-byte segments) and staged with rows of 32 C + 4 floats, so neither the global reads nor the shared stores serialise.
+template <int C, bool TRANS>
+__device__ __forceinline__ int small_w_index(int idx, int& kr, int& c) {
+  if (!TRANS) {
+    kr = idx / (32 * C); c = idx - kr * 32 * C;
+    return idx;
+  }
+  const int lo = idx & 31, hi = idx >> 5;
+  kr = (lo & 7) + 8 * (hi & 3); c = (lo >> 3) + 4 * (hi >> 2);
+  return kr * (32 * C + 4) + c;
+}
+template <int C, bool TRANS = false>
 __device__ __forceinline__ void small_w_fetch(float (&pre)[kSmallKT * C / 8], const float* __restrict__ W, int ldw, int K, int N, int k0) {
-  constexpr int LDW = 32 * C;
 #pragma unroll
   for (int i = 0; i < kSmallKT * C / 8; ++i) {
-    const int idx = threadIdx.x + kSmallThreads * i, kr = idx / LDW, c = idx - kr * LDW;
-    pre[i] = (k0 + kr < K && c < N) ? __ldg(W + (size_t)(k0 + kr) * ldw + c) : 0.f;
+    int kr, c;
+    small_w_index<C, TRANS>(threadIdx.x + kSmallThreads * i, kr, c);
+    pre[i] = (k0 + kr < K && c < N) ? __ldg(TRANS ? W + (size_t)c * ldw + k0 + kr : W + (size_t)(k0 + kr) * ldw + c) : 0.f;
   }
 }
-template <int C>
+template <int C, bool TRANS = false>
 __device__ __forceinline__ void small_w_store(const float (&pre)[kSmallKT * C / 8], float* Ws) {
 #pragma unroll
-  for (int i = 0; i < kSmallKT * C / 8; ++i) Ws[threadIdx.x + kSmallThreads * i] = pre[i];
+  for (int i = 0; i < kSmallKT * C / 8; ++i) {
+    int kr, c;
+    Ws[small_w_index<C, TRANS>(threadIdx.x + kSmallThreads * i, kr, c)] = pre[i];
+  }
 }
+// staging floats of one k-tile (two are double-buffered in Wst)
+template <int C, bool TRANS>
+__host__ __device__ constexpr int small_w_tile() { return kSmallKT * (TRANS ? 32 * C + 4 : 32 * C); }
 
-template <int R, int C, class Epi>
+template <int R, int C, bool TRANS, class Epi>
 __device__ __forceinline__ void small_gemm_r(const float* X, int ldx, int M, int K, const float* __restrict__ W, int ldw, int N,
                                              float* Wst, const Epi& epi) {
-  constexpr int LDW = 32 * C;
-  static_assert((kSmallKT * LDW) % kSmallThreads == 0, "whole tile per thread");
+  constexpr int LDW = TRANS ? 32 * C + 4 : 32 * C, TILE = small_w_tile<C, TRANS>();
+  static_assert((kSmallKT * 32 * C) % kSmallThreads == 0, "whole tile per thread");
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r0 = warp * R;
   const bool active = r0 < M;
@@ -97,13 +116,13 @@ __device__ __forceinline__ void small_gemm_r(const float* X, int ldx, int M, int
   }
   const int ntile = (K + kSmallKT - 1) / kSmallKT;
   float pre[kSmallKT * C / 8];
-  small_w_fetch<C>(pre, W, ldw, K, N, 0);
-  small_w_store<C>(pre, Wst);
+  small_w_fetch<C, TRANS>(pre, W, ldw, K, N, 0);
+  small_w_store<C, TRANS>(pre, Wst);
   __syncthreads();
   for (int t = 0; t < ntile; ++t) {
-    if (t + 1 < ntile) small_w_fetch<C>(pre, W, ldw, K, N, (t + 1) * kSmallKT);
+    if (t + 1 < ntile) small_w_fetch<C, TRANS>(pre, W, ldw, K, N, (t + 1) * kSmallKT);
     if (active) {
-      const float* Ws = Wst + (t & 1) * (kSmallKT * LDW) + lane * C;
+      const float* Ws = Wst + (t & 1) * TILE + lane * C;
       const int k0 = t * kSmallKT, rows = imin(kSmallKT, K - k0);
       int kk = 0;
       for (; kk + 4 <= rows; kk += 4) {
@@ -134,7 +153,7 @@ __device__ __forceinline__ void small_gemm_r(const float* X, int ldx, int M, int
         }
       }
     }
-    if (t + 1 < ntile) small_w_store<C>(pre, Wst + ((t + 1) & 1) * (kSmallKT * LDW));
+    if (t + 1 < ntile) small_w_store<C, TRANS>(pre, Wst + ((t + 1) & 1) * TILE);
     __syncthreads();
   }
   if (!active) return;
@@ -149,48 +168,50 @@ __device__ __forceinline__ void small_gemm_r(const float* X, int ldx, int M, int
 template <int C, class Epi>
 __device__ __forceinline__ void small_gemm(const float* X, int ldx, int M, int K, const float* __restrict__ W, int ldw, int N,
                                            float* Wst, const Epi& epi) {
-  if (M <= kSmallWarps) small_gemm_r<1, C>(X, ldx, M, K, W, ldw, N, Wst, epi);
-  else if (M <= 2 * kSmallWarps) small_gemm_r<2, C>(X, ldx, M, K, W, ldw, N, Wst, epi);
-  else small_gemm_r<4, C>(X, ldx, M, K, W, ldw, N, Wst, epi);
+  if (M <= kSmallWarps) small_gemm_r<1, C, false>(X, ldx, M, K, W, ldw, N, Wst, epi);
+  else if (M <= 2 * kSmallWarps) small_gemm_r<2, C, false>(X, ldx, M, K, W, ldw, N, Wst, epi);
+  else small_gemm_r<4, C, false>(X, ldx, M, K, W, ldw, N, Wst, epi);
+}
+// Y = epi(X.W^T): the same product with W [N][ldw] in Keras layout read transposed (K = its row length used); Wst holds
+// 2 small_w_tile<C, true>() floats
+template <int C, class Epi>
+__device__ __forceinline__ void small_gemm_t(const float* X, int ldx, int M, int K, const float* __restrict__ W, int ldw, int N,
+                                             float* Wst, const Epi& epi) {
+  if (M <= kSmallWarps) small_gemm_r<1, C, true>(X, ldx, M, K, W, ldw, N, Wst, epi);
+  else if (M <= 2 * kSmallWarps) small_gemm_r<2, C, true>(X, ldx, M, K, W, ldw, N, Wst, epi);
+  else small_gemm_r<4, C, true>(X, ldx, M, K, W, ldw, N, Wst, epi);
 }
 
-__global__ void __launch_bounds__(kSmallThreads) k_tower_forward(const TowerFwdArgs a) {
-  SPW_DYN_SMEM(smem_raw);
-  __shared__ int s_bad;
+// Node state the backward pass (k_tower_backward, spw_small_grad.cuh) takes from the forward: per node, kNodeState floats
+// at these offsets (step l of G / U at + kDP l, of P at + kDP (l - 1), of S / R at + 2 kDEP (l - 1); p^0 = S^0 = R^0 = 0 are
+// not stored).
+constexpr int kNsQ1 = 0, kNsQ = kDP, kNsG = 2 * kDP, kNsP = 7 * kDP, kNsU = 11 * kDP, kNsS = 16 * kDP, kNsZ = kNsS + 8 * kDEP;
+constexpr int kNodeState = kNsZ + 4;
+
+// 1 if tower [n0, n0 + nt) must not be computed: edges outside the tower or the edge arrays, offsets going backwards (a
+// malformed graph must not index out of bounds).  eb, ee: its in-edge rows.  Every thread of the CTA calls it (barriers inside).
+__device__ __forceinline__ int tower_malformed(const TowerFwdArgs& a, int n0, int nt, int eb, int ee, int* s_bad) {
   const int tid = threadIdx.x;
-  const int n0 = a.node_off[blockIdx.x], nt = a.node_off[blockIdx.x + 1] - n0;
-  if (nt <= 0) return;
-  const float qnan = nanf("");
-  if (nt > a.max_nodes) {                     // larger than the caller declared: this tower's rows are NaN, nothing else is written
-    for (int i = tid; i < nt; i += kSmallThreads) {
-      a.logits[n0 + i] = qnan;
-      if (a.probs) a.probs[n0 + i] = qnan;
-    }
-    return;
-  }
-  const int eb = a.in_off[n0], ee = a.in_off[n0 + nt], ne = ee - eb;
-  // a malformed graph (edges outside the tower or the edge arrays, offsets going backwards) must not index out of bounds
-  if (tid == 0) s_bad = (eb < 0 || ee > a.n_edges || ne < 0) ? 1 : 0;
+  if (tid == 0) *s_bad = (eb < 0 || ee > a.n_edges || ee < eb) ? 1 : 0;
   __syncthreads();
-  if (!s_bad) {
+  if (!*s_bad) {
     for (int e = eb + tid; e < ee; e += kSmallThreads) {
       const int s = a.in_snd[e], r = a.in_rcv[e];
-      if (s < n0 || s >= n0 + nt || r < n0 || r >= n0 + nt) s_bad = 1;
+      if (s < n0 || s >= n0 + nt || r < n0 || r >= n0 + nt) *s_bad = 1;
     }
     for (int i = tid; i < nt; i += kSmallThreads)
-      if (a.in_off[n0 + i] > a.in_off[n0 + i + 1]) s_bad = 1;
+      if (a.in_off[n0 + i] > a.in_off[n0 + i + 1]) *s_bad = 1;
   }
   __syncthreads();
-  if (s_bad) {
-    for (int i = tid; i < nt; i += kSmallThreads) {
-      a.logits[n0 + i] = qnan;
-      if (a.probs) a.probs[n0 + i] = qnan;
-    }
-    return;
-  }
+  return *s_bad;
+}
 
+// The forward pass of tower [n0, n0 + nt) with in-edge rows [eb, eb + ne), in shared memory `sm` (small_smem_layout): the
+// logit of each block goes to a.logits (and a.probs) when they are set.  save != null: the node state of kNodeState floats
+// per block (kNs*) is also written there, for the backward pass; the arithmetic is the same either way.
+__device__ __forceinline__ void tower_forward_body(const TowerFwdArgs& a, float* sm, int n0, int nt, int eb, int ne, float* save) {
+  const int tid = threadIdx.x;
   const SmallSmem L = small_smem_layout(a.max_nodes);
-  float* sm = reinterpret_cast<float*>(smem_raw);
   float* QV = sm + L.QV;
   float* GP = sm + L.GP;
   float* U = sm + L.U;
@@ -217,6 +238,13 @@ __global__ void __launch_bounds__(kSmallThreads) k_tower_forward(const TowerFwdA
   small_gemm<4>(U, kDP, nt, kDP, w.om_w[1], kDP, kDP,
                 Wst, [&](int r, int c, float v) { GP[r * 2 * kDP + c] = relu_f(v + __ldg(w.om_b[1] + c)); });
   __syncthreads();
+  if (save) {                                 // q1 (in U) and q (in the g half of GP), both complete at the barrier above
+    for (int idx = tid; idx < nt * kDP; idx += kSmallThreads) {
+      const int i = idx / kDP, c = idx - i * kDP;
+      save[(size_t)i * kNodeState + kNsQ1 + c] = U[i * kDP + c];
+      save[(size_t)i * kNodeState + kNsQ + c] = GP[i * 2 * kDP + c];
+    }
+  }
   // qv = q.V1a + c1: the object-encoding part of omp layer 0, the same in all five steps (Networks.py:89)
   small_gemm<4>(GP, 2 * kDP, nt, kDP, w.omp_w[0], kDP, kDP,
                 Wst, [&](int r, int c, float v) { QV[r * kDP + c] = v + __ldg(w.omp_b[0] + c); });
@@ -294,6 +322,22 @@ __global__ void __launch_bounds__(kSmallThreads) k_tower_forward(const TowerFwdA
     small_gemm<4>(GP, 2 * kDP, nt, l == 0 ? kDP : 2 * kDP, V1bc, kDP, kDP,
                   Wst, [&](int r, int c, float v) { U[r * kDP + c] = relu_f(QV[r * kDP + c] + v); });
     __syncthreads();
+    if (save) {                  // g^l, p^l, u^l, S^l, R^l: read here, before the p update below writes p^{l+1}
+      for (int idx = tid; idx < nt * kDP; idx += kSmallThreads) {
+        const int i = idx / kDP, c = idx - i * kDP;
+        float* sv = save + (size_t)i * kNodeState;
+        sv[kNsG + l * kDP + c] = GP[i * 2 * kDP + c];
+        sv[kNsU + l * kDP + c] = U[i * kDP + c];
+        if (l > 0) sv[kNsP + (l - 1) * kDP + c] = GP[i * 2 * kDP + kDP + c];
+      }
+      if (l > 0)
+        for (int idx = tid; idx < nt * kDE; idx += kSmallThreads) {
+          const int i = idx / kDE, c = idx - i * kDE;
+          float* sv = save + (size_t)i * kNodeState + kNsS + (l - 1) * 2 * kDEP;
+          sv[c] = S[i * kDEP + c];
+          sv[kDEP + c] = Rr[i * kDEP + c];
+        }
+    }
     if (l < SPW_N_STEPS - 1) {   // p = tanh(z[1:] + p)   (Networks.py:80,91); the update after the last step is dead
       small_gemm<4>(U, kDP, nt, kDP, w.omp_w[1] + 1, kDP + 1, kDP, Wst, [&](int r, int c, float v) {
         float* p = GP + r * 2 * kDP + kDP + c;
@@ -307,9 +351,29 @@ __global__ void __launch_bounds__(kSmallThreads) k_tower_forward(const TowerFwdA
     float s = 0.f;
     for (int k = 0; k < kDP; ++k) s = fmaf(U[i * kDP + k], __ldg(w.omp_w[1] + (size_t)k * (kDP + 1)), s);
     const float z = s + __ldg(w.omp_b[1]);
-    a.logits[n0 + i] = z;
+    if (a.logits) a.logits[n0 + i] = z;
+    if (save) save[(size_t)i * kNodeState + kNsZ] = z;
     if (a.probs) a.probs[n0 + i] = 1.f / (1.f + expf(-z));
   }
+}
+
+__global__ void __launch_bounds__(kSmallThreads) k_tower_forward(const TowerFwdArgs a) {
+  SPW_DYN_SMEM(smem_raw);
+  __shared__ int s_bad;
+  const int tid = threadIdx.x;
+  const int n0 = a.node_off[blockIdx.x], nt = a.node_off[blockIdx.x + 1] - n0;
+  if (nt <= 0) return;
+  const float qnan = nanf("");
+  const int eb = nt > a.max_nodes ? 0 : a.in_off[n0], ee = nt > a.max_nodes ? 0 : a.in_off[n0 + nt];
+  // larger than the caller declared, or malformed: this tower's rows are NaN, nothing else is written
+  if (nt > a.max_nodes || tower_malformed(a, n0, nt, eb, ee, &s_bad)) {
+    for (int i = tid; i < nt; i += kSmallThreads) {
+      a.logits[n0 + i] = qnan;
+      if (a.probs) a.probs[n0 + i] = qnan;
+    }
+    return;
+  }
+  tower_forward_body(a, reinterpret_cast<float*>(smem_raw), n0, nt, eb, ee - eb, nullptr);
 }
 
 }  // namespace spw

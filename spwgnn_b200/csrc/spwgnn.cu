@@ -11,6 +11,7 @@
 #include "spw_csl_kernels.cuh"
 #include "spw_csl_wgrad.cuh"
 #include "spw_small.cuh"
+#include "spw_small_grad.cuh"
 #include "spw_obj_grad.cuh"
 #include "spw_rel_grad.cuh"
 #include "spw_input_grad.cuh"
@@ -1151,6 +1152,45 @@ int spw_forward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_
   set_smem(k_tower_forward, smem);
   SPW_KLAUNCH("k_tower_forward", k_tower_forward, dim3(g->n_towers), dim3(kSmallThreads), smem, (cudaStream_t)stream, a);
   return check_launch("spw_forward_towers");
+}
+
+size_t spw_backward_towers_bytes(int32_t n_nodes, int32_t n_edges) {
+  if (n_nodes < 0 || n_edges < 0) return 0;
+  return small_bwd_ws_floats(n_nodes, n_edges) * sizeof(float);   // A_e, d A_e, the node state of every step
+}
+
+int spw_backward_towers(const SpwParams* w, const SpwGraph* g, int32_t max_nodes_per_tower, const float* obj,
+                        const float* dlogits, const float* dprobs, float* logits, float* dobj, float* drel,
+                        void* workspace, size_t workspace_bytes, void* stream) {
+  int rc;
+  if ((rc = check_params(w, "spw_backward_towers")) != SPW_OK) return rc;
+  if ((rc = check_graph(g)) != SPW_OK) return rc;
+  if (max_nodes_per_tower < 0) return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: negative max_nodes_per_tower");
+  if (max_nodes_per_tower > SPW_SMALL_MAX_NODES)
+    return fail(SPW_ERR_UNSUPPORTED, "spw_backward_towers: %d blocks in a tower, limit is %d", max_nodes_per_tower, SPW_SMALL_MAX_NODES);
+  const int n = g->n_nodes, E = g->n_edges;
+  if (n == 0 || g->n_towers == 0) return SPW_OK;
+  if (!obj || !dobj) return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: null pointer");
+  if (!dlogits && !dprobs) return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: null seed (dlogits and dprobs both null)");
+  if (!aligned16(obj) || !aligned16(dobj) || (logits && !aligned16(logits)))
+    return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: obj, dobj or logits not 16-byte aligned");
+  if (reinterpret_cast<uintptr_t>(drel) % sizeof(float) || reinterpret_cast<uintptr_t>(dlogits) % sizeof(float) ||
+      reinterpret_cast<uintptr_t>(dprobs) % sizeof(float))
+    return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: dlogits, dprobs or drel not 4-byte aligned");
+  const size_t need = spw_backward_towers_bytes(n, E);
+  if (workspace_bytes < need) return fail(SPW_ERR_WORKSPACE, "spw_backward_towers: workspace %zu < %zu bytes", workspace_bytes, need);
+  if (!workspace || !aligned16(workspace)) return fail(SPW_ERR_BAD_ARG, "spw_backward_towers: workspace null or not 16-byte aligned");
+  float* ws = reinterpret_cast<float*>(workspace);
+  TowerBwdArgs a;
+  a.f.w = *w; a.f.node_off = g->node_off; a.f.in_off = g->in_off; a.f.in_snd = g->in_snd; a.f.in_rcv = g->in_rcv; a.f.obj = obj;
+  a.f.logits = logits; a.f.probs = nullptr; a.f.A = ws; a.f.n_edges = E;
+  a.f.max_nodes = max_nodes_per_tower > 0 ? max_nodes_per_tower : 1;
+  a.out_off = g->out_off; a.out_pos = g->out_pos; a.dlogits = dlogits; a.dprobs = dprobs; a.dobj = dobj;
+  a.drel = E > 0 ? drel : nullptr; a.dA = ws + (size_t)E * kDEP; a.ns = ws + (size_t)2 * E * kDEP;
+  const size_t smem = small_bwd_smem_bytes(a.f.max_nodes);
+  set_smem(k_tower_backward, smem);
+  SPW_KLAUNCH("k_tower_backward", k_tower_backward, dim3(g->n_towers), dim3(kSmallThreads), smem, (cudaStream_t)stream, a);
+  return check_launch("spw_backward_towers");
 }
 
 int spw_bce_grad(const float* logits, const float* target, int32_t n_nodes, double count, float* dlogits, double* stats,

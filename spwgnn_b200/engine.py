@@ -145,6 +145,40 @@ class Engine:
                                                  ws.data_ptr(), ws.numel(), _stream_ptr(self.device)))
         return logits[:n], (probs[:n] if want_probs else None)
 
+    def gradients_towers(self, batch: TowerBatch, dlogits=None, dprobs=None, want_drel=False):
+        """The backward pass of forward_towers in ONE kernel launch (spw_backward_towers): the logits and the gradient of
+        sum(dlogits*logits + dprobs*sigmoid(logits)) with respect to the block features and, with want_drel, the relation
+        weights, for towers of at most SMALL_MAX_NODES blocks.  dlogits, dprobs: (n_nodes,) tensors on this device, either
+        may be None, not both.  Returns (logits (n,), dobj (n, 3), drel (n_edges,) or None) on the device: logits are
+        forward_towers' bits, dobj / drel are what relation_gradients computes (to fp32 rounding), and a tower's results are
+        the same bits whatever else is in the batch.  Uses ws_small, so a training step in flight is left alone."""
+        if batch.max_nodes > SMALL_MAX_NODES:
+            raise SpwError('gradients_towers: towers of up to %d blocks, this batch allows %d' % (SMALL_MAX_NODES, batch.max_nodes))
+        if dlogits is None and dprobs is None:
+            raise SpwError('gradients_towers: give dlogits, dprobs or both')
+        api, n, E = self.api, batch.n_nodes, batch.n_edges
+
+        def seed(t, name):
+            if t is None:
+                return None
+            t = t.detach().to(torch.float32).contiguous()
+            if t.shape != (n,) or t.device.type != 'cuda' or (self.device.index is not None and t.device.index != self.device.index):
+                raise SpwError('gradients_towers: %s must be (%d,) on %s, got %s on %s' % (name, n, self.device, tuple(t.shape), t.device))
+            return t
+        dl, dp = seed(dlogits, 'dlogits'), seed(dprobs, 'dprobs')
+        with torch.cuda.device(self.device):
+            logits = torch.empty(max(n, 1), dtype=torch.float32, device=self.device)
+            dobj = torch.empty(max(n, 1), 3, dtype=torch.float32, device=self.device)
+            drel = torch.empty(max(E, 1), dtype=torch.float32, device=self.device) if want_drel else None
+            ws = self.ws_small.get(api.dll.spw_backward_towers_bytes(n, E))
+            wp = self.params.c_struct()
+            api.check(api.dll.spw_backward_towers(ctypes.byref(wp), ctypes.byref(batch.c_graph), int(batch.max_nodes),
+                                                  batch.obj.data_ptr(), None if dl is None else dl.data_ptr(),
+                                                  None if dp is None else dp.data_ptr(), logits.data_ptr(), dobj.data_ptr(),
+                                                  drel.data_ptr() if want_drel and E else None, ws.data_ptr(), ws.numel(),
+                                                  _stream_ptr(self.device)))
+        return logits[:n], dobj[:n], (drel[:E] if want_drel else None)
+
     # ---- loss seed + backward -------------------------------------------------------------------
     def bce_seed(self, logits, target, count):
         """Keras binary_crossentropy (Networks.py:102).  Returns (dlogits, stats) with stats a device
